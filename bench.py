@@ -2,7 +2,7 @@
 """bench.py -- torque-feasibility states/s (Panda 7-DOF RNE) on N B200s, with the roofline of the
 dominant kernel, an end-to-end number through the host-buffer C-ABI call, and the CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -20,6 +20,10 @@ Timing (same at every N): W warm-up steps, then the step is held for ~1 s so eve
 (power-capped) clock regime, then EXACTLY K steps -- captured once into one CUDA graph per rank, so the timed
 region is K back-to-back kernels, not K Python launches -- between a barrier + synchronize on both sides,
 CUDA events on the launching stream, max over ranks.
+
+--dump-outputs DIR (N = 1) writes what the last timed step returned, so two builds can be compared output for
+output on the same seeded inputs: DIR/tau.npy (float64 [7][1M] joint torques) and DIR/feasible.npy (the uint8
+mask [1M] as float32), 60 MB in all.
 
 --impl reference times the CPU implementation of the same path on the host cores: the reference's
 rne.py is pure Python/NumPy and cannot travel to the GPU box, so this arm runs the C oracle port of
@@ -454,8 +458,14 @@ def main():
                     help="N > 1: how the feasibility masks are all-gathered each step: p2p = peer stores fused into the "
                          "torque kernel (tcmp_rne_batch_scatter) + completion flags (tcmp_peer_signal / tcmp_peer_wait) on "
                          "a side stream; nccl = all_gather_into_tensor on a side stream")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs as DIR/tau.npy and DIR/feasible.npy (N = 1 only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the GPU path, not --impl reference")
         return run_reference(args)
 
     import torch
@@ -469,6 +479,8 @@ def main():
         raise SystemExit("bench.py needs a B200: the product path has no CPU fallback")
     all_cores, affinity = bind_rank_to_cores(local, world)
     torch.cuda.set_device(local)
+    if world > 1 and args.dump_outputs:
+        raise SystemExit("--dump-outputs needs a single-GPU run")
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     dev = torch.device("cuda", local)
@@ -613,6 +625,8 @@ def main():
     timed(main_run)                  # first replay of a graph uploads it (~0.1 ms): not part of a step
     settle_reps, _ = hold(hold200, args.settle_s)
     ms_total = timed(main_run)       # the contract's number: exactly K timed steps
+    # the outputs of timed step K - 1, copied before the runs below overwrite the buffers
+    dumped = (out_tau.clone(), out_mask.clone()) if args.dump_outputs else None
     # sustained rate over >= 1.5 s, and the kernel alone (no gather epilogue, no wait) over the same >= 200 launches
     # at every N for the roofline of the dominant kernel
     sus_reps, sus_ms = hold(hold200, 1.5)
@@ -859,6 +873,10 @@ def main():
                                                        "300 states on one core"}
             if world == 1 and not args.no_extras:
                 out["cpu_baseline"]["other_workloads"] = cpu_baseline_extras()
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "tau.npy"), dumped[0].cpu().numpy())
+            np.save(os.path.join(args.dump_outputs, "feasible.npy"), dumped[1].cpu().numpy().astype(np.float32))
         print(json.dumps(out))
     if world > 1:
         dist.barrier()

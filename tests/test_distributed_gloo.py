@@ -10,6 +10,7 @@ import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
+import ik_reference as ref
 import oracle
 from conftest import sample_edges, sample_states
 
@@ -33,7 +34,7 @@ def _oracle_edge(qa, qb, W, mass, mode="rne", **kw):
 
 def _oracle_ik(r, t, f):
     n = lambda a: a.numpy() if torch.is_tensor(a) else a
-    sols, counts = oracle.ref_ik_batch(n(r), n(t), n(f))
+    sols, counts, _ = ref.host_ik(n(r), n(t), n(f))
     return torch.as_tensor(sols), torch.as_tensor(counts)
 
 
@@ -50,14 +51,13 @@ def _worker(rank, world, port, n_states, n_edges, n_poses, q):
         qa, qb = sample_edges(n_edges, seed=4)
         ff, _ = D.sharded_edge_feasibility(qa, qb, 16, 5.0, compute=_oracle_edge)
         assert np.array_equal(ff.numpy(), oracle.edge_feasibility("rne", qa, qb, 16, 5.0))
-        if oracle.have_ref():
-            rng = np.random.default_rng(3)
-            qq = rng.uniform(-2.5, 2.5, size=(7, n_poses)); qq[3] = -np.abs(qq[3]) - 0.1; qq[5] = np.abs(qq[5])
-            trans, rot = oracle.ref_fk_batch(qq)
-            free = np.stack([qq[6], rng.uniform(-2.8, 2.8, n_poses)])
-            sols, counts, _ = D.sharded_ik(rot, trans, free, compute=_oracle_ik)
-            s_full, c_full = oracle.ref_ik_batch(rot, trans, free)
-            assert np.array_equal(counts.numpy(), c_full) and np.array_equal(sols.numpy(), s_full)
+        rng = np.random.default_rng(3)
+        qq = rng.uniform(-2.5, 2.5, size=(7, n_poses)); qq[3] = -np.abs(qq[3]) - 0.1; qq[5] = np.abs(qq[5])
+        trans, rot = ref.fk_batch(qq)
+        free = np.stack([qq[6], rng.uniform(-2.8, 2.8, n_poses)])
+        sols, counts, _ = D.sharded_ik(rot, trans, free, compute=_oracle_ik)
+        s_full, c_full, _ = ref.host_ik(rot, trans, free)
+        assert np.array_equal(counts.numpy(), c_full) and np.array_equal(sols.numpy(), s_full)
         q.put((rank, "ok"))
     except Exception as e:  # pragma: no cover
         q.put((rank, repr(e)))

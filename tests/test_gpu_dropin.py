@@ -6,6 +6,7 @@ import random
 import numpy as np
 import pytest
 
+import ik_reference as ref
 import oracle
 from conftest import Q_HI, Q_LO, load_golden, sample_states
 
@@ -69,9 +70,8 @@ def test_remaining_reference_named_helpers():
     assert len(I) == 10 and np.allclose(np.diag(I[9]), [2.0 * 0.165 ** 2, 2.0 * 0.165 ** 2, 0.0])
     R.remove_payload()
     pose = ikfast.ikfast_forward_kinematics(None, ikfast.PANDA_INFO, None, Q_HOME)
-    if oracle.have_ref():
-        trans, rot = oracle.ref_fk_batch(np.asarray(Q_HOME, dtype=float).reshape(7, 1))
-        assert np.abs(np.asarray(pose[0]) - trans[:, 0]).max() < 1e-12
+    trans, rot = ref.fk_batch(np.asarray(Q_HOME, dtype=float).reshape(7, 1))
+    assert np.abs(np.asarray(pose[0]) - trans[:, 0]).max() < 1e-12
     assert ikfast.check_solution(None, list(range(7)), Q_HOME, None, pose)
     moved = list(Q_HOME); moved[1] += 0.01
     assert not ikfast.check_solution(None, list(range(7)), moved, None, pose)
@@ -126,9 +126,9 @@ def test_special_poses_counts_on_gpu():
     rng = np.random.default_rng(6)
     n = 50_000
     q = np.clip(rng.choice(vals, size=(7, n)), Q_LO[:, None], Q_HI[:, None])
-    trans, rot = oracle.ref_fk_batch(q)
+    trans, rot = ref.fk_batch(q)
     free = np.stack([q[6], rng.choice(vals, size=n)])
-    _, cr = oracle.ref_ik_batch(rot, trans, free, want_sols=False)
+    _, cr = ref.ik_batch("special_value_poses_50k", rot, trans, free, want_sols=False)
     _, c, st = engine.ik_batch(rot, trans, free, want_sols=False)
     # singular poses: the count can hinge on a 1e-6 / 5e-6 threshold met to the last ulp, where CUDA's libm
     # and FMA contraction differ from glibc; report and bound the disagreement instead of hiding it

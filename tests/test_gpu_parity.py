@@ -9,6 +9,7 @@ import math
 import numpy as np
 import pytest
 
+import ik_reference as ref
 import oracle
 from conftest import load_golden, sample_edges, sample_states
 
@@ -292,19 +293,18 @@ def test_ik_vs_reference_golden(eng):
 
 def test_ik_round_trip_100k(eng):
     """FK(IK(pose)) == pose for every returned solution (the reference's own self-check idea,
-    ikfast.py:93-102, tolerance 1e-6), and counts match the compiled reference on 100k x 3 solves."""
+    ikfast.py:93-102, tolerance 1e-6), and counts match the reference on 100k x 3 solves."""
     import torch
     rng = np.random.default_rng(33)
     n = 100_000
     from conftest import Q_HI, Q_LO
     q = rng.uniform(Q_LO[:, None], Q_HI[:, None], size=(7, n))
-    trans, rot = eng.fk_batch(dev(q))
+    trans_h, rot_h = ref.fk_batch(q)
+    trans, rot = dev(trans_h), dev(rot_h)
     free = np.stack([q[6], rng.uniform(-2.8973, 2.8973, n), rng.uniform(-2.8973, 2.8973, n)])
     sols, counts, status = eng.ik_batch(rot, trans, dev(free))
-    _, counts_ref = oracle.ref_ik_batch(rot.cpu().numpy(), trans.cpu().numpy(), free, want_sols=False)
     cnt = counts.cpu().numpy()
-    mism = np.nonzero(cnt != counts_ref)[0]
-    assert len(mism) == 0, (len(mism), mism[:10], cnt[mism[:10]], counts_ref[mism[:10]])
+    ref.check("round_trip_100k", cnt, sols.cpu().numpy(), inputs=(rot_h, trans_h, free), tol=1e-9)
     assert (cnt.reshape(n, 3)[:, 0] >= 1).all()          # the pose's own j7 always yields a solution
     # round trip on the valid slots
     valid = (torch.arange(8, device="cuda")[None, :] < counts[:, None])
@@ -354,16 +354,16 @@ def test_scatter_kernel_single_rank(eng):
 
 
 def test_ik_select_vs_composed_reference(eng):
-    """tcmp_ik_select == reference IK (compiled) -> joint-limit filter (ikfast.py:167) -> static torque test
+    """tcmp_ik_select == reference IK -> joint-limit filter (ikfast.py:167) -> static torque test
     (oracle) -> nearest to the current configuration (max norm, ikfast.py:172-188), composed on the CPU."""
     from conftest import Q_HI, Q_LO
     rng = np.random.default_rng(44)
     n, nf = 3000, 6
     q = rng.uniform(Q_LO[:, None], Q_HI[:, None], size=(7, n))
-    trans, rot = oracle.ref_fk_batch(q)
+    trans, rot = ref.fk_batch(q)
     free = np.vstack([q[6:7], rng.uniform(Q_LO[6], Q_HI[6], size=(nf - 1, n))])
     q_ref = np.clip(q + rng.normal(0, 0.4, size=q.shape), Q_LO[:, None], Q_HI[:, None])
-    sols, counts = oracle.ref_ik_batch(rot, trans, free)
+    sols, counts = ref.ik_batch("select_composed", rot, trans, free)
     for mode, mass, norm in [("rne", 5.0, "inf"), ("nov", 3.0, "l2"), ("base", 0.0, "inf"), ("dyn", 4.0, "inf")]:
         best, cost, nv = eng.ik_select(rot, trans, free, q_ref, mass, mode=mode, norm=norm)
         exp_cost = np.full(n, np.inf)
@@ -463,12 +463,12 @@ def test_ik_select_sweep_longer_than_a_warp(eng):
     n, nf = 600, 40
     q = rng.uniform(Q_LO[:, None] + 1e-6, Q_HI[:, None] - 1e-6, size=(7, n))
     q[5] = np.minimum(q[5], 3.1)      # the solver returns angles wrapped to (-pi, pi]: joint 6 above pi would come back
-    trans, rot = oracle.ref_fk_batch(q)   # as q - 2 pi, outside its limits, and be filtered like the reference does
+    trans, rot = ref.fk_batch(q)          # as q - 2 pi, outside its limits, and be filtered like the reference does
     free = np.vstack([rng.uniform(Q_LO[6], Q_HI[6], size=(nf - 1, n)), q[6:7]])     # the exact j7 comes LAST
     best, cost, nv = eng.ik_select(rot, trans, free, q, 0.0, mode="base", norm="inf")
     # the pose's own configuration is reachable with cost ~ 0 and lives in the second round
     assert (cost < 1e-9).all() and np.abs(best - q).max() < 1e-9 and (nv >= 1).all()
-    sols, counts = oracle.ref_ik_batch(rot, trans, free)
+    sols, counts = ref.ik_batch("select_sweep_40", rot, trans, free)
     inside = ((sols >= Q_LO) & (sols <= Q_HI)).all(axis=2) & (np.arange(8)[None, :] < counts[:, None])
     assert np.array_equal(nv, inside.reshape(n, nf, 8).sum(axis=(1, 2)).astype(np.int32))
 
@@ -587,10 +587,10 @@ def test_model_ik_select_and_extend_prefix(eng):
     rng = np.random.default_rng(72)
     n, nf = 1500, 5
     q = rng.uniform(Q_LO[:, None], Q_HI[:, None], size=(7, n))
-    trans, rot = oracle.ref_fk_batch(q)
+    trans, rot = ref.fk_batch(q)
     free = np.vstack([q[6:7], rng.uniform(Q_LO[6], Q_HI[6], size=(nf - 1, n))])
     q_ref = np.clip(q + rng.normal(0, 0.4, size=q.shape), Q_LO[:, None], Q_HI[:, None])
-    sols, counts = oracle.ref_ik_batch(rot, trans, free)
+    sols, counts = ref.ik_batch("select_model", rot, trans, free)
     best, cost, nv = eng.ik_select(rot, trans, free, q_ref, 3.0, mode="rne", model=model)
     exp_cost, exp_nv = np.full(n, np.inf), np.zeros(n, dtype=np.int32)
     cand, owner = [], []

@@ -1,6 +1,6 @@
 """CPU: host-side logic of the drop-in layer (no GPU): min-jerk coefficients vs the reference's golden
 vectors, extend/refine/distance helpers, batched vs serial safe_path, RRT* against the reference's own
-rrt_star_force_aware (imported read-only when /root/reference exists), pose algebra, collision stand-in.
+rrt_star_force_aware (imported read-only from $TCMP_REFERENCE_SRC, the original's src/ directory, when set), pose algebra, collision stand-in.
 The torque predicate in these tests is the CPU oracle -- the thing being tested is the host logic."""
 import math
 import os
@@ -15,7 +15,8 @@ from conftest import Q_HI, Q_LO, load_golden
 
 from torque_constrained_motion_planning_b200 import collision, ik_utils, min_jerk_v2, panda_model, rrt_star, utils
 
-HAVE_REF = os.path.exists("/root/reference/src/rrt_star.py")
+REF_SRC = os.environ.get("TCMP_REFERENCE_SRC", "")
+HAVE_REF = os.path.exists(os.path.join(REF_SRC, "rrt_star.py"))
 
 
 def oracle_torque_fn(mass, mode="rne"):
@@ -88,11 +89,11 @@ def test_rrt_star_matches_reference_tree_growth(seed):
     """Same seeds, same predicates -> the batched RRT* returns exactly what the reference's
     rrt_star_force_aware returns (strict_reference mode)."""
     sys.dont_write_bytecode = True
-    if "/root/reference/src" not in sys.path:
-        sys.path.insert(0, "/root/reference/src")
+    if REF_SRC not in sys.path:
+        sys.path.insert(0, REF_SRC)
     import importlib
     ref = importlib.import_module("rrt_star")
-    assert ref.__file__.startswith("/root/reference")
+    assert ref.__file__.startswith(REF_SRC)
 
     joints = list(range(7))
     res = 0.1 * np.ones(7)
@@ -175,11 +176,10 @@ def test_collision_stand_in():
     assert col(down)
     qs = np.random.default_rng(3).uniform(Q_LO, Q_HI, size=(200, 7))
     assert np.array_equal(col.batch(qs), np.array([col(q) for q in qs]))
-    # link frames agree with the reference FK (ikfast ComputeFk) at the flange
-    if oracle.have_ref():
-        o = collision.link_frames(qs)
-        trans, _ = oracle.ref_fk_batch(np.ascontiguousarray(qs.T))
-        assert np.abs(o[:, 7].T - trans).max() < 1e-12
+    # link frames agree with the reference FK (ikfast ComputeFk, golden poses) at the flange
+    g = load_golden("ik_cfg3.npz")
+    o = collision.link_frames(np.ascontiguousarray(g["q"].T))
+    assert np.abs(o[:, 7].T - g["trans"]).max() < 1e-12
 
 
 def test_problem_and_panda_model_surface():

@@ -126,16 +126,18 @@ def test_dyn_defined_oracle_consistency():
     t2, _ = oracle.torque_test_batch("dyn", q, qd, qdd, 2.0)
     t4, _ = oracle.torque_test_batch("dyn", q, qd, qdd, 4.0)
     assert np.abs((t4 - t0) - 2 * (t2 - t0)).max() < 1e-10
-    if oracle.have_ref():
-        # d(height of tool)/dq_i * m g == J^T F; tool = link8 origin + 0.105 along its z axis
-        def tool_z(qq):
-            tr_, rot = oracle.ref_fk_batch(qq)
-            return tr_[2] + 0.105 * rot[8]
-        h = 1e-6
-        for i in range(7):
-            dq = np.zeros((7, 1)); dq[i] = h
-            num = (tool_z(q + dq) - tool_z(q - dq)) / (2 * h) * 2.0 * 9.81
-            assert np.abs(num - (t2 - t0)[i]).max() < 1e-6
+    # d(height of tool)/dq_i * m g == J^T F; tool = link8 origin + 0.105 along its z axis (FK of ComputeFk's
+    # convention, checked against the reference's golden poses in test_ik_core_host)
+    import ik_reference
+
+    def tool_z(qq):
+        tr_, rot = ik_reference.fk_batch(qq)
+        return tr_[2] + 0.105 * rot[8]
+    h = 1e-6
+    for i in range(7):
+        dq = np.zeros((7, 1)); dq[i] = h
+        num = (tool_z(q + dq) - tool_z(q - dq)) / (2 * h) * 2.0 * 9.81
+        assert np.abs(num - (t2 - t0)[i]).max() < 1e-6
 
 
 def test_ref_ikfast_kats():
