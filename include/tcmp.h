@@ -103,6 +103,29 @@ int tcmp_rne_batch_model(const tcmp_model *model, int mode, int dtype, int64_t n
                          double payload_threshold, void *tau_out, uint8_t *feasible_out, void *stream);
 
 /*
+ * Joint-space dynamics terms of the model tcmp_rne_batch evaluates, fp64, per state -- what the reference's `dyn`
+ * test imports from panda_dynamics_model (get_mass_matrix / get_coriolis_matrix / get_gravity_vector,
+ * panda_primitives.py:86-91) plus the tool Jacobian it takes from PyBullet (:93-99):
+ *   g_out [7][n]     g(q) = rne(q, 0, 0)
+ *   M_out [7][7][n]  joint-space inertia matrix, element (r, c) of state i at (r*7 + c)*n + i; exactly symmetric
+ *   C_out [7][7][n]  Christoffel-consistent Coriolis matrix C_ij = sum_k Gamma_ijk qd_k: C qd = rne(q, qd, 0) - g
+ *                    and Mdot = C + C^T
+ *   J_out [6][7][n]  geometric Jacobian of the grasp-target point (link-7 origin + (0, 0, 0.107 + tool_z)) in the
+ *                    base frame, rows [linear; angular]
+ * so that M qdd + C qd + g == tcmp_rne_batch(TCMP_MODE_RNE, ..., TCMP_PAYLOAD_THRESHOLD_RAW).
+ *   model         host pointer or NULL (compiled-in Panda).
+ *   q [7][n]; qd [7][n], required iff C_out != NULL.
+ *   payload_mass  [n] or NULL (then payload_scalar): a rigid body on the flange iff m > 0 (rne.py:184); 0 gives the
+ *                 arm alone, as panda_dynamics_model does.
+ * Each output may be NULL (not computed); at least one is required when n > 0.  n == 0 returns TCMP_OK whatever the
+ * buffers (an empty array may have a NULL data pointer).  Enqueues only: no allocation, no synchronisation, so the
+ * call can be captured in a CUDA graph.
+ */
+int tcmp_dynamics_batch(const tcmp_model *model, int64_t n, const double *q, const double *qd,
+                        const double *payload_mass, double payload_scalar, double *M_out, double *C_out,
+                        double *g_out, double *J_out, void *stream);
+
+/*
  * Multi-GPU form of tcmp_rne_batch: the feasibility byte of state i is stored into dest_masks[d][dest_offset + i]
  * for every d < n_dest -- the gathered mask buffers of all ranks (this rank's own and its peers', mapped with
  * tcmp_peer_open over NVLink/NVSwitch).  This is the "NCCL all-gather of the masks" of BASELINE.json's

@@ -203,6 +203,21 @@ int tcmp_rne_batch_model(const tcmp_model *model, int mode, int dtype, int64_t n
     return TCMP_OK;
 }
 
+int tcmp_dynamics_batch(const tcmp_model *model, int64_t n, const double *q, const double *qd,
+                        const double *payload_mass, double payload_scalar, double *M_out, double *C_out, double *g_out,
+                        double *J_out, void *stream) {
+    if (n < 0) return fail(TCMP_ERR_INVALID_ARG, "negative count %lld", (long long)n);
+    if (int rc = check_model(model)) return rc;
+    // an empty batch is a no-op whatever the buffers (empty arrays may have NULL data pointers), as in tcmp_rne_batch
+    if (n == 0) return TCMP_OK;
+    if (!q) return fail(TCMP_ERR_INVALID_ARG, "q is NULL");
+    if (!M_out && !C_out && !g_out && !J_out) return fail(TCMP_ERR_INVALID_ARG, "every output is NULL");
+    if (C_out && !qd) return fail(TCMP_ERR_INVALID_ARG, "C_out needs qd");
+    TCMP_CUDA(launch_dynamics_batch(model, n, q, qd, payload_mass, payload_scalar, M_out, C_out, g_out, J_out,
+                                    (cudaStream_t)stream));
+    return TCMP_OK;
+}
+
 int tcmp_rne_batch_scatter(int mode, int dtype, int64_t n, const void *q, const void *qd, const void *qdd,
                            const void *payload_mass, double payload_scalar, double payload_threshold, void *tau_out,
                            int n_dest, void *const *dest_masks, int64_t dest_offset, void *stream) {

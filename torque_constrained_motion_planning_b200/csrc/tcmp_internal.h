@@ -43,6 +43,11 @@ cudaError_t launch_rne_batch_model(const tcmp_model &model, int mode, int dtype,
 void default_model_desc(tcmp_model *out);
 const char *model_desc_problem(const tcmp_model &model);
 
+// dynamics_kernels.cu: M, C, g, J per state (any output may be NULL; model NULL = compiled-in Panda)
+cudaError_t launch_dynamics_batch(const tcmp_model *model, int64_t n, const double *q, const double *qd,
+                                  const double *payload_mass, double payload_scalar, double *M_out, double *C_out,
+                                  double *g_out, double *J_out, cudaStream_t st);
+
 // Per-rank sync block of the fused gathers (TCMP_PEER_SYNC_BYTES, allocated with tcmp_peer_alloc, zeroed once):
 // arrived[r] = last epoch rank r has published here (written by rank r's kernels over NVLink); epoch / ticket are
 // this rank's own.

@@ -492,6 +492,37 @@ def fk_batch(q):
     return trans, rot
 
 
+def dynamics_batch(q, qd=None, payload_mass=0.0, mass_matrix: bool = True, coriolis: bool = False,
+                   gravity: bool = True, jacobian: bool = False, model: Optional[InertialModel] = None):
+    """Joint-space dynamics terms per state (tcmp_dynamics_batch), fp64: q ``[7][n]``, qd ``[7][n]`` (needed for the
+    Coriolis matrix), payload_mass scalar or ``[n]`` (a rigid body on the flange iff m > 0; 0 = the arm alone).
+    Returns ``{"M": [7][7][n], "C": [7][7][n], "g": [7][n], "J": [6][7][n]}`` with None for the terms not requested;
+    M qdd + C qd + g equals the rne torques.  J is the geometric Jacobian [linear; angular] of the grasp-target point
+    in the base frame.  CUDA tensors in -> CUDA tensors out, NumPy in -> NumPy out."""
+    if not (mass_matrix or coriolis or gravity or jacobian):
+        raise ValueError("nothing to compute")
+    if coriolis and qd is None:
+        raise ValueError("the Coriolis matrix needs qd")
+    torch = _torch()
+    lib = load()
+    host = not _is_cuda_tensor(q)
+    dev = torch.device("cuda", torch.cuda.current_device()) if host else q.device
+    n = int(q.shape[1])
+    scalar, pm = (float(payload_mass), None) if np.ndim(payload_mass) == 0 else (0.0, payload_mass)
+    with torch.cuda.device(dev):
+        qt = _as_dev(q, "f64", (7, n), dev)
+        qdt = _as_dev(qd, "f64", (7, n), dev) if coriolis else None
+        pmt = _as_dev(pm, "f64", (n,), dev)
+        mk = lambda want, shape: torch.empty(shape, dtype=torch.float64, device=dev) if want else None
+        out = {"M": mk(mass_matrix, (7, 7, n)), "C": mk(coriolis, (7, 7, n)), "g": mk(gravity, (7, n)),
+               "J": mk(jacobian, (6, 7, n))}
+        check(lib.tcmp_dynamics_batch(_mptr(model), n, _ptr(qt), _ptr(qdt), _ptr(pmt), scalar, _ptr(out["M"]),
+                                      _ptr(out["C"]), _ptr(out["g"]), _ptr(out["J"]), _stream_ptr()))
+    if host:
+        return {k: None if v is None else v.cpu().numpy() for k, v in out.items()}
+    return out
+
+
 def fp64_peak(iters: int = 4096) -> float:
     """Measured FP64 FMA throughput of the current device in FLOP/s (tcmp_fp64_peak)."""
     out = ctypes.c_double(0.0)
