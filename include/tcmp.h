@@ -278,7 +278,9 @@ int tcmp_fk_batch(int64_t n, const double *q, double *trans3, double *rot9, void
  * Synthetic-scene collision predicate (stand-in for utils.get_collision_fn, utils.py:3165-3218, whose PyBullet
  * backend is out of scope): joint-limit test first (utils.py:3177-3178), then link spheres from the DH forward
  * kinematics against axis-aligned boxes / spheres.  Obstacle and limit arrays are HOST memory (copied into the
- * launch parameters).  hit_out[i] = 1 when configuration i collides or violates a joint limit.
+ * launch parameters).  hit_out[i] = 1 when configuration i collides or violates a joint limit.  As in the NumPy
+ * stand-in (collision.get_collision_fn), a NaN joint passes the limit test and the link spheres it moves hit nothing;
+ * a +-inf joint is outside any finite limit.
  */
 #define TCMP_MAX_OBSTACLES 32
 typedef struct {

@@ -17,7 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtcmp.so")
 SOURCES = ["rne_kernels.cu", "model_kernels.cu", "edge_kernels.cu", "ik_kernels.cu", "select_kernels.cu", "collision_kernels.cu", "dynamics_kernels.cu", "tcmp_api.cu"]
-HEADERS = ["panda_model.cuh", "dynamics_core.cuh", "ik_core.cuh", "sincos_table.inc", "tcmp_internal.h", os.path.join("..", "..", "include", "tcmp.h")]
+HEADERS = ["panda_model.cuh", "collision_core.cuh", "dynamics_core.cuh", "ik_core.cuh", "sincos_table.inc", "tcmp_internal.h", os.path.join("..", "..", "include", "tcmp.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

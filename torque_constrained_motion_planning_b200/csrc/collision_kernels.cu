@@ -24,83 +24,12 @@ static __device__ const SinCos kExtSinCosTable[kSinCosTableSize] = {
 #include "sincos_table.inc"
 };
 
-struct Scene {
-    int n_obs;
-    int kind[TCMP_MAX_OBSTACLES];            // 0 = box, 1 = sphere
-    double c[TCMP_MAX_OBSTACLES][3];         // centre
-    double h[TCMP_MAX_OBSTACLES][3];         // box half extents; sphere: h[0] = radius
-    double lo[7], hi[7];                     // joint limits (limits_fn, utils.py:3177)
-    double payload_radius;                   // > 0: a sphere at the grasp target (held object)
-};
+}  // namespace tcmp
 
-// Link-sphere model of collision.py (_SEGMENTS): spheres strung between consecutive DH frame origins
-// 1..7 and the grasp target (8).
-__device__ constexpr int kSegCount = 7;
-__device__ constexpr int kSegSamples[kSegCount] = {3, 2, 4, 2, 2, 2, 3};
-__device__ constexpr double kSegRadius[kSegCount] = {0.07, 0.07, 0.065, 0.06, 0.055, 0.05, 0.05};
+// Included after kExtSinCosTable so that the table keeps the first slot of the kernels' global-address constant bank.
+#include "collision_core.cuh"
 
-__device__ __forceinline__ bool sphere_hits(const Scene &S, double x, double y, double z, double r) {
-    bool hit = false;
-    for (int o = 0; o < S.n_obs; ++o) {
-        const double dx = x - S.c[o][0], dy = y - S.c[o][1], dz = z - S.c[o][2];
-        if (S.kind[o] == 1) {
-            hit = hit || (sqrt(dx * dx + dy * dy + dz * dz) < r + S.h[o][0]);
-        } else {
-            const double ex = fmax(fabs(dx) - S.h[o][0], 0.0), ey = fmax(fabs(dy) - S.h[o][1], 0.0),
-                         ez = fmax(fabs(dz) - S.h[o][2], 0.0);
-            hit = hit || (sqrt(ex * ex + ey * ey + ez * ez) < r);
-        }
-    }
-    return hit;
-}
-
-// collision.py get_collision_fn.batch for one configuration
-__device__ bool config_collides(const Scene &S, const double (&q)[7]) {
-    bool out = false;
-#pragma unroll
-    for (int j = 0; j < 7; ++j) out = out || (q[j] < S.lo[j]) || (q[j] > S.hi[j]);
-    if (out || S.n_obs == 0) return out;
-    // origins of DH frames 0..7 and the grasp target (collision.link_frames)
-    double O[9][3];
-    double X[3] = {1, 0, 0}, Y[3] = {0, 1, 0}, Z[3] = {0, 0, 1}, p[3] = {0, 0, 0};
-    const double A[7] = {0, 0, 0, 0.0825, -0.0825, 0, 0.088};
-    const double D[7] = {0.333, 0, 0.316, 0, 0.384, 0, 0};
-    const int AL[7] = {0, -1, 1, 1, -1, 1, 1};
-#pragma unroll
-    for (int k = 0; k < 7; ++k) {
-        double s, c;
-        sincos(q[k], &s, &c);
-#pragma unroll
-        for (int r = 0; r < 3; ++r) {
-            const double y = AL[k] == 0 ? Y[r] : (AL[k] > 0 ? Z[r] : -Z[r]);
-            const double z = AL[k] == 0 ? Z[r] : (AL[k] > 0 ? -Y[r] : Y[r]);
-            p[r] += A[k] * X[r] + D[k] * z;
-            const double x = X[r];
-            X[r] = c * x + s * y;
-            Y[r] = c * y - s * x;
-            Z[r] = z;
-            O[k][r] = p[r];
-        }
-    }
-#pragma unroll
-    for (int r = 0; r < 3; ++r) {
-        O[7][r] = p[r] + 0.107 * Z[r];
-        O[8][r] = O[7][r] + 0.105 * Z[r];
-    }
-    bool hit = false;
-#pragma unroll
-    for (int g = 0; g < kSegCount; ++g) {
-        const int a = g + 1, b = g + 2, m = kSegSamples[g];
-        for (int i = 0; i < m; ++i) {
-            const double t = (double)i / (double)(m - 1);   // np.linspace(0, 1, m)
-            const double x = (1 - t) * O[a][0] + t * O[b][0], y = (1 - t) * O[a][1] + t * O[b][1],
-                         z = (1 - t) * O[a][2] + t * O[b][2];
-            hit = hit || sphere_hits(S, x, y, z, kSegRadius[g]);
-        }
-    }
-    if (S.payload_radius > 0) hit = hit || sphere_hits(S, O[8][0], O[8][1], O[8][2], S.payload_radius);
-    return hit;
-}
+namespace tcmp {
 
 __global__ void __launch_bounds__(128)
 collision_kernel(int64_t n, const double *__restrict__ q, Scene S, uint8_t *__restrict__ hit_out) {
@@ -132,30 +61,15 @@ extend_prefix_kernel(int64_t n_edges, const double *__restrict__ q1, const doubl
         for (int j = 0; j < 7; ++j) {
             a[j] = __ldg(q1 + j * n_edges + e);
             b[j] = __ldg(q2 + j * n_edges + e);
-            const double d = __ddiv_rn(__dadd_rn(b[j], -a[j]), res[j]);   // np.divide(difference, resolutions)
-            nrm2 = __dadd_rn(nrm2, __dmul_rn(d, d));
+            nrm2 = extend_norm2_add(nrm2, a[j], b[j], res[j]);
         }
-        // steps = int(np.linalg.norm(., ord=2)) (utils.py:3074); the sequence has steps + 1 configurations
-        // A non-finite norm (NaN / inf end point) has no step count: report 0 configurations, safe prefix 0, so the
-        // host never truncates a sequence with it (the cast of a NaN to int is undefined); a huge finite norm is
-        // clamped for the same reason.
-        const double nrm = sqrt(nrm2);
-        const bool sane = nrm == nrm && nrm < 1.0e6;
-        const int N = sane ? (int)nrm + 1 : 0;
+        const int N = extend_num_configs(nrm2);   // 0 for a non-finite or huge norm
         int prefix = N;
         for (int base = 0; base < N; base += 32) {
             const int k = base + lane;
             const bool active = k < N;
-            // get_refine_fn recurrence (utils.py:3036-3039): q <- (1 / (N - i)) * (q2 - q) + q, i = 0..k
             double q[7];
-#pragma unroll
-            for (int j = 0; j < 7; ++j) q[j] = a[j];
-            const int last = active ? k : N - 1;
-            for (int i = 0; i <= last; ++i) {
-                const double w = __ddiv_rn(1.0, (double)(N - i));
-#pragma unroll
-                for (int j = 0; j < 7; ++j) q[j] = __dadd_rn(__dmul_rn(w, __dadd_rn(b[j], -q[j])), q[j]);
-            }
+            extend_config(a, b, N, active ? k : N - 1, q);
             bool bad = config_collides(S, q);
             if (!bad && check_torque) {   // torque only for collision-free configurations (rrt_star.py:92-96)
                 double tau[7];
@@ -179,19 +93,7 @@ extend_prefix_kernel(int64_t n_edges, const double *__restrict__ q1, const doubl
 static cudaError_t make_scene(int n_obs, const tcmp_obstacle *obs, const double *q_lo, const double *q_hi,
                               double payload_radius, Scene *S) {
     if (n_obs < 0 || n_obs > TCMP_MAX_OBSTACLES) return cudaErrorInvalidValue;
-    S->n_obs = n_obs;
-    for (int o = 0; o < TCMP_MAX_OBSTACLES; ++o) {
-        S->kind[o] = o < n_obs ? obs[o].kind : 0;
-        for (int r = 0; r < 3; ++r) {
-            S->c[o][r] = o < n_obs ? obs[o].center[r] : 0.0;
-            S->h[o][r] = o < n_obs ? obs[o].half[r] : 0.0;
-        }
-    }
-    for (int j = 0; j < 7; ++j) {
-        S->lo[j] = q_lo[j];
-        S->hi[j] = q_hi[j];
-    }
-    S->payload_radius = payload_radius;
+    fill_scene(n_obs, obs, q_lo, q_hi, payload_radius, S);
     return cudaSuccess;
 }
 
