@@ -69,6 +69,9 @@ int tcmp_device_count(void);
  *   payload_threshold  payload attached iff mass > threshold (rne/nov); dyn applies the
  *                   mass unconditionally as a tool-point force (panda_primitives.py:101-110).
  *   tau_out         [7][n] or NULL;  feasible_out [n] (1 = within limits) or NULL.
+ * A NaN or infinite joint angle -- joint 1's too, although its value cannot change a torque -- gives NaN torques
+ * and, since NaN never compares >= a limit, a feasible verdict, as rne.py does.  The edge, trajectory, IK-select
+ * and extend-prefix torque tests follow the same rule.
  */
 int tcmp_rne_batch(int mode, int dtype, int64_t n, const void *q, const void *qd, const void *qdd,
                    const void *payload_mass, double payload_scalar, double payload_threshold,
@@ -113,6 +116,8 @@ int tcmp_rne_batch_model(const tcmp_model *model, int mode, int dtype, int64_t n
  *   J_out [6][7][n]  geometric Jacobian of the grasp-target point (link-7 origin + (0, 0, 0.107 + tool_z)) in the
  *                    base frame, rows [linear; angular]
  * so that M qdd + C qd + g == tcmp_rne_batch(TCMP_MODE_RNE, ..., TCMP_PAYLOAD_THRESHOLD_RAW).
+ * M, C and g do not read joint 1's angle: a NaN or infinite q[0] leaves them finite (and J NaN), where
+ * tcmp_rne_batch returns NaN torques.
  *   model         host pointer or NULL (compiled-in Panda).
  *   q [7][n]; qd [7][n], required iff C_out != NULL.
  *   payload_mass  [n] or NULL (then payload_scalar): a rigid body on the flange iff m > 0 (rne.py:184); 0 gives the

@@ -479,10 +479,16 @@ TCMP_FN bool sincos6_table(const double (&q)[7], double (&s)[7], double (&c)[7],
     return true;
 }
 
-// The recursion proper, given sin / cos of joints 2..7 (s[0], c[0] are never read).
+// Gravity as rne_core applies it: g + 0 * q[0].  The product is +-0 for a finite joint-1 angle, so the value is g
+// exactly, and NaN for a NaN or infinite one.  Joint 1's angle cannot change a torque, but the reference rotates
+// by it (rne.py), so a non-finite q[0] gives it NaN torques -- and, since NaN never compares >= a limit, a feasible
+// verdict.  Folding q[0] into the base acceleration makes every torque here NaN in the same cases (one FMA).
+template <typename T> TCMP_FN T gravity_for(T q0) { return q0 * T(0) + T(kGravity); }
+
+// The recursion proper, given sin / cos of joints 2..7 (s[0], c[0] are never read) and the gravity magnitude.
 template <typename T, bool DYN, bool TOOL, typename P = ConstParams>
 TCMP_FN void rne_body(const T (&s)[7], const T (&c)[7], const T (&qd)[7], const T (&qdd)[7], T mp_inertial,
-                      T mp_tool, T (&tau)[7], const P &p = P()) {
+                      T mp_tool, T (&tau)[7], const P &p = P(), T gravity = T(kGravity)) {
 
     V3<T> F[7], N[7];
     Kin<T> k;
@@ -495,7 +501,7 @@ TCMP_FN void rne_body(const T (&s)[7], const T (&c)[7], const T (&qd)[7], const 
         k.w = {-s[1] * qd[0], -c[1] * qd[0], qd[1]};
         k.wd = {-s[1] * qdd[0] + k.w.y * qd[1], -c[1] * qdd[0] - k.w.x * qd[1], qdd[1]};
     }
-    k.vd = {-s[1] * T(kGravity), -c[1] * T(kGravity), T(0)};
+    k.vd = {-s[1] * gravity, -c[1] * gravity, T(0)};
     if constexpr (TOOL && DYN) gv = k.vd;
     link_wrench_const<1, T, DYN>(p, k, F[1], N[1]);
 
@@ -556,7 +562,7 @@ TCMP_FN void rne_core(const T (&q)[7], const T (&qd)[7], const T (&qdd)[7], T mp
                       const P &p = P()) {
     T c[7], s[7];
     sincos6<T>(q, s, c);
-    rne_body<T, DYN, TOOL, P>(s, c, qd, qdd, mp_inertial, mp_tool, tau, p);
+    rne_body<T, DYN, TOOL, P>(s, c, qd, qdd, mp_inertial, mp_tool, tau, p, gravity_for(q[0]));
 }
 
 // K1's form: sin / cos from the table (shared-memory copy, or GLOBAL = in place) when every angle allows it.
@@ -568,7 +574,7 @@ TCMP_FN void rne_core_table(const double (&q)[7], const double (&qd)[7], const d
 #pragma unroll
         for (int j = 1; j < 7; ++j) sincos_t<double>(q[j], &s[j], &c[j]);
     }
-    rne_body<double, DYN, TOOL, P>(s, c, qd, qdd, mp_inertial, mp_tool, tau, p);
+    rne_body<double, DYN, TOOL, P>(s, c, qd, qdd, mp_inertial, mp_tool, tau, p, gravity_for(q[0]));
 }
 
 // |tau_i| < limit_i for i in 0..5 (panda_primitives.py:182-183; joint 7 is never tested).
