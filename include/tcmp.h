@@ -131,6 +131,49 @@ int tcmp_dynamics_batch(const tcmp_model *model, int64_t n, const double *q, con
                         double *g_out, double *J_out, void *stream);
 
 /*
+ * Payload-mass intervals: which payload masses a state, or every waypoint of an RRT* edge, can carry within the torque
+ * limits -- the inverse of the torque test, in one launch (a bisection over the mass takes ~26 torque-test launches to
+ * reach 1e-6 kg over [0, 64] kg, and is wrong when the passing masses do not start at 0: a payload can pull a joint's
+ * torque back inside its limit).  fp64 only.
+ *
+ * Every joint torque of the torque test is affine in the mass: tau(m) = a + m b for every mass the test attaches
+ * (m > payload_threshold in rne / nov, every m in dyn).  For one state (q, qd, qdd) and mode:
+ *   a [7]  the torque with no payload (mp_inertial = mp_tool = 0);
+ *   b [7]  the torque one kilogram adds: rne / nov, the payload rigid body on link 7 (unit mass, axial first moment
+ *          0.107, jxx = jyy = payload_radius^2 + 0.107^2, everything else 0); dyn, the tool-point gravity force (moment
+ *          arm 0.107 + tool_z).  One forward Newton-Euler pass, a's backward pass, and b's (one wrench carried down).
+ * Per joint j in 0..5 (joint 7 is never tested) the passing masses are the open interval {m : |a_j + m b_j| < L_j}:
+ *   b_j > 0: ((-L_j - a_j) / b_j, (L_j - a_j) / b_j); b_j < 0: the ends swap;
+ *   b_j == 0: (-inf, +inf) if |a_j| < L_j, else the empty (+inf, -inf);
+ *   a_j or b_j NaN: (-inf, +inf) -- NaN never compares >= a limit, so the torque test passes the joint at every mass.
+ * Outputs per state:
+ *   m_lo = max over joints of the lower ends, m_hi = min of the upper ends, over all real m (either may be negative);
+ *     the interval is empty iff m_lo >= m_hi.
+ *   unloaded_ok = |a_j| < L_j for j = 0..5: the verdict with no payload attached.
+ * Contract: for every mass the torque test attaches, its verdict is m_lo < m < m_hi; for a mass it does not attach it
+ * is unloaded_ok -- except where some torque lies within 1e-9 N.m of a limit (the torque contract).  So the payload
+ * threshold is not an input here: engine.payload_passes / engine.max_payload apply it.
+ * A NaN or infinite joint angle (joint 1's too) makes every torque NaN: (-inf, +inf) and unloaded_ok = 1, as
+ * tcmp_rne_batch judges such a state feasible at every mass.  TCMP_MODE_BASE writes (-inf, +inf, 1) and reads no input.
+ *   model   host pointer or NULL (compiled-in Panda), as in tcmp_dynamics_batch.
+ *   q, qd, qdd [7][n]: qd / qdd both given or both NULL (= static), ignored in TCMP_MODE_NOV; q may be NULL in BASE.
+ *   m_lo_out, m_hi_out [n] double, unloaded_ok_out [n]: each may be NULL, at least one is required when n > 0.
+ * n == 0 returns TCMP_OK whatever the buffers.  Bad mode, n < 0, n_waypoints < 1 or a missing q return
+ * TCMP_ERR_INVALID_ARG before any CUDA call.  Enqueues only (no allocation, no synchronisation): graph-capturable.
+ *
+ * tcmp_edge_payload_interval: per edge qa -> qb, the intersection over its n_waypoints min-jerk samples, which are
+ * exactly tcmp_edge_feasibility's (t = linspace(1/W, 1, W); static_only tests (q, 0, 0)): max of m_lo, min of m_hi,
+ * AND of unloaded_ok.  Exact, so an edge's result means what a state's does: tcmp_edge_feasibility(..., m) returns
+ * n_waypoints iff m lies in the edge's interval (or, for an unattached m, iff unloaded_ok).
+ */
+int tcmp_payload_interval_batch(const tcmp_model *model, int mode, int64_t n, const double *q, const double *qd,
+                                const double *qdd, double *m_lo_out, double *m_hi_out, uint8_t *unloaded_ok_out,
+                                void *stream);
+int tcmp_edge_payload_interval(const tcmp_model *model, int mode, int64_t n_edges, int n_waypoints,
+                               const double *qa, const double *qb, int static_only, double *m_lo_out,
+                               double *m_hi_out, uint8_t *unloaded_ok_out, void *stream);
+
+/*
  * Multi-GPU form of tcmp_rne_batch: the feasibility byte of state i is stored into dest_masks[d][dest_offset + i]
  * for every d < n_dest -- the gathered mask buffers of all ranks (this rank's own and its peers', mapped with
  * tcmp_peer_open over NVLink/NVSwitch).  This is the "NCCL all-gather of the masks" of BASELINE.json's

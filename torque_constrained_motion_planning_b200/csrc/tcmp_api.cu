@@ -218,6 +218,39 @@ int tcmp_dynamics_batch(const tcmp_model *model, int64_t n, const double *q, con
     return TCMP_OK;
 }
 
+static int check_payload_common(const tcmp_model *model, int mode, int64_t n) {
+    if (mode < TCMP_MODE_RNE || mode > TCMP_MODE_BASE) return fail(TCMP_ERR_INVALID_ARG, "bad mode %d", mode);
+    if (n < 0) return fail(TCMP_ERR_INVALID_ARG, "negative count %lld", (long long)n);
+    return check_model(model);
+}
+
+int tcmp_payload_interval_batch(const tcmp_model *model, int mode, int64_t n, const double *q, const double *qd,
+                                const double *qdd, double *m_lo_out, double *m_hi_out, uint8_t *unloaded_ok_out,
+                                void *stream) {
+    if (int rc = check_payload_common(model, mode, n)) return rc;
+    if (n == 0) return TCMP_OK;
+    if (!q && mode != TCMP_MODE_BASE) return fail(TCMP_ERR_INVALID_ARG, "q is NULL");
+    if (!m_lo_out && !m_hi_out && !unloaded_ok_out) return fail(TCMP_ERR_INVALID_ARG, "every output is NULL");
+    if ((qd == nullptr) != (qdd == nullptr))
+        return fail(TCMP_ERR_INVALID_ARG, "qd and qdd must both be given or both be NULL");
+    TCMP_CUDA(launch_payload_interval(model, mode, n, q, qd, qdd, m_lo_out, m_hi_out, unloaded_ok_out,
+                                      (cudaStream_t)stream));
+    return TCMP_OK;
+}
+
+int tcmp_edge_payload_interval(const tcmp_model *model, int mode, int64_t n_edges, int n_waypoints, const double *qa,
+                               const double *qb, int static_only, double *m_lo_out, double *m_hi_out,
+                               uint8_t *unloaded_ok_out, void *stream) {
+    if (int rc = check_payload_common(model, mode, n_edges)) return rc;
+    if (n_waypoints < 1) return fail(TCMP_ERR_INVALID_ARG, "n_waypoints must be >= 1");
+    if (n_edges == 0) return TCMP_OK;
+    if ((!qa || !qb) && mode != TCMP_MODE_BASE) return fail(TCMP_ERR_INVALID_ARG, "NULL edge buffer");
+    if (!m_lo_out && !m_hi_out && !unloaded_ok_out) return fail(TCMP_ERR_INVALID_ARG, "every output is NULL");
+    TCMP_CUDA(launch_edge_payload_interval(model, mode, n_edges, n_waypoints, qa, qb, static_only, m_lo_out, m_hi_out,
+                                           unloaded_ok_out, (cudaStream_t)stream));
+    return TCMP_OK;
+}
+
 int tcmp_rne_batch_scatter(int mode, int dtype, int64_t n, const void *q, const void *qd, const void *qdd,
                            const void *payload_mass, double payload_scalar, double payload_threshold, void *tau_out,
                            int n_dest, void *const *dest_masks, int64_t dest_offset, void *stream) {

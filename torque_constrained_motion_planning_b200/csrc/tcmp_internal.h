@@ -48,6 +48,15 @@ cudaError_t launch_dynamics_batch(const tcmp_model *model, int64_t n, const doub
                                   const double *payload_mass, double payload_scalar, double *M_out, double *C_out,
                                   double *g_out, double *J_out, cudaStream_t st);
 
+// payload_kernels.cu: payload-mass intervals per state (K11) and per min-jerk edge (K12); each output may be NULL,
+// mode BASE fills (-inf, +inf, 1) and reads nothing; model NULL = compiled-in Panda
+cudaError_t launch_payload_interval(const tcmp_model *model, int mode, int64_t n, const double *q, const double *qd,
+                                    const double *qdd, double *m_lo_out, double *m_hi_out, uint8_t *unloaded_ok_out,
+                                    cudaStream_t st);
+cudaError_t launch_edge_payload_interval(const tcmp_model *model, int mode, int64_t n_edges, int n_waypoints,
+                                         const double *qa, const double *qb, int static_only, double *m_lo_out,
+                                         double *m_hi_out, uint8_t *unloaded_ok_out, cudaStream_t st);
+
 // Per-rank sync block of the fused gathers (TCMP_PEER_SYNC_BYTES, allocated with tcmp_peer_alloc, zeroed once):
 // arrived[r] = last epoch rank r has published here (written by rank r's kernels over NVLink); epoch / ticket are
 // this rank's own.

@@ -523,6 +523,121 @@ def dynamics_batch(q, qd=None, payload_mass=0.0, mass_matrix: bool = True, corio
     return out
 
 
+def _interval_outputs(torch, n, dev):
+    return (torch.empty((n,), dtype=torch.float64, device=dev), torch.empty((n,), dtype=torch.float64, device=dev),
+            torch.empty((n,), dtype=torch.uint8, device=dev))
+
+
+def payload_interval_batch(q, qd=None, qdd=None, mode: str = "rne", model: Optional[InertialModel] = None):
+    """Payload masses each state can carry within the torque limits (tcmp_payload_interval_batch), fp64.
+    q/qd/qdd ``[7][n]`` (qd/qdd both or neither; ignored in nov).  Returns ``(m_lo [n], m_hi [n], unloaded_ok uint8
+    [n])``: the torque test at an attached mass m passes iff m_lo < m < m_hi, and with no payload attached iff
+    unloaded_ok (see :func:`payload_passes`, :func:`max_payload`).  CUDA tensors in -> CUDA tensors out, NumPy in ->
+    NumPy out."""
+    if (qd is None) != (qdd is None):
+        raise ValueError("qd and qdd must both be given or both be None")
+    torch = _torch()
+    lib = load()
+    host = not _is_cuda_tensor(q)
+    dev = torch.device("cuda", torch.cuda.current_device()) if host else q.device
+    n = int(q.shape[1])
+    dynamic = mode != "nov" and qd is not None
+    with torch.cuda.device(dev):
+        qt = _as_dev(q, "f64", (7, n), dev)
+        qdt = _as_dev(qd, "f64", (7, n), dev) if dynamic else None
+        qddt = _as_dev(qdd, "f64", (7, n), dev) if dynamic else None
+        lo, hi, ok = _interval_outputs(torch, n, dev)
+        check(lib.tcmp_payload_interval_batch(_mptr(model), MODE[mode], n, _ptr(qt), _ptr(qdt), _ptr(qddt), _ptr(lo),
+                                              _ptr(hi), _ptr(ok), _stream_ptr()))
+    if host:
+        return lo.cpu().numpy(), hi.cpu().numpy(), ok.cpu().numpy()
+    return lo, hi, ok
+
+
+def edge_payload_interval(qa, qb, n_waypoints: int = 64, mode: str = "rne", static_only: bool = False,
+                          model: Optional[InertialModel] = None):
+    """Payload masses each RRT* edge qa -> qb can carry at every one of its min-jerk waypoints (the samples of
+    :func:`edge_feasibility`), per edge (tcmp_edge_payload_interval).  qa/qb ``[7][n_edges]``.  Returns
+    ``(m_lo, m_hi, unloaded_ok)`` as :func:`payload_interval_batch`; edge_feasibility at an attached mass m returns
+    n_waypoints iff m_lo < m < m_hi."""
+    torch = _torch()
+    lib = load()
+    host = not _is_cuda_tensor(qa)
+    dev = torch.device("cuda", torch.cuda.current_device()) if host else qa.device
+    n = int(qa.shape[1])
+    with torch.cuda.device(dev):
+        a = _as_dev(qa, "f64", (7, n), dev)
+        b = _as_dev(qb, "f64", (7, n), dev)
+        lo, hi, ok = _interval_outputs(torch, n, dev)
+        check(lib.tcmp_edge_payload_interval(_mptr(model), MODE[mode], n, int(n_waypoints), _ptr(a), _ptr(b),
+                                             int(static_only), _ptr(lo), _ptr(hi), _ptr(ok), _stream_ptr()))
+    if host:
+        return lo.cpu().numpy(), hi.cpu().numpy(), ok.cpu().numpy()
+    return lo, hi, ok
+
+
+def traj_payload_interval(coeffs, samples_per_segment: int, mode: str = "rne", model: Optional[InertialModel] = None,
+                          device=None):
+    """Payload masses a whole piecewise min-jerk trajectory (coefficients ``[n_seg][7][6]``) can carry: the
+    intersection over the samples :func:`traj_feasibility` tests.  Returns ``(m_lo, m_hi, unloaded_ok)`` as Python
+    float, float, int; traj_feasibility at an attached mass m finds no failure iff m_lo < m < m_hi."""
+    torch = _torch()
+    if mode == "base":
+        return -float("inf"), float("inf"), 1
+    s = traj_feasibility(coeffs, samples_per_segment, mode="base", want_tau=False, device=device, model=model)
+    lo, hi, ok = payload_interval_batch(s["q"], s["qd"], s["qdd"], mode=mode, model=model)
+    if lo.numel() == 0:
+        return -float("inf"), float("inf"), 1
+    r = torch.stack([lo.max(), hi.min(), ok.min().to(torch.float64)]).cpu().tolist()
+    return r[0], r[1], int(r[2])
+
+
+def _xp(x):
+    """torch for tensors, NumPy for everything else (the interval helpers work on either)."""
+    import sys
+    torch = sys.modules.get("torch")
+    return torch if torch is not None and torch.is_tensor(x) else np
+
+
+def max_payload(m_lo, m_hi, unloaded_ok, mode: str, payload_threshold: float = PAYLOAD_THRESHOLD_TEST):
+    """Elementwise: the largest M such that the torque test passes at every mass in [0, M), from the intervals of
+    :func:`payload_interval_batch` / :func:`edge_payload_interval` (torch tensors or NumPy arrays).
+      rne / nov: masses up to the threshold are not attached, so 0 if the unloaded arm fails, else m_hi when
+                 m_lo <= threshold < m_hi and the threshold otherwise;
+      dyn:       the tool force applies at every mass: max(m_hi, 0) when unloaded_ok and m_lo <= 0, else 0;
+      base:      +inf."""
+    xp = _xp(m_lo)
+    hi = m_hi if xp is not np else np.asarray(m_hi, dtype=np.float64)
+    lo = m_lo if xp is not np else np.asarray(m_lo, dtype=np.float64)
+    ok = (unloaded_ok if xp is not np else np.asarray(unloaded_ok)) != 0
+    zero = xp.zeros_like(hi)
+    if mode == "base":
+        return xp.full_like(hi, float("inf"))
+    if mode == "dyn":
+        return xp.where(ok & (lo <= 0), xp.where(hi > 0, hi, zero), zero)
+    t = float(payload_threshold)
+    return xp.where(ok, xp.where((lo <= t) & (t < hi), hi, xp.full_like(hi, t)), zero)
+
+
+def payload_passes(m_lo, m_hi, unloaded_ok, mass, mode: str, payload_threshold: float = PAYLOAD_THRESHOLD_TEST):
+    """Elementwise: the torque test's verdict at payload mass ``mass`` (scalar or per element), reproduced from the
+    intervals -- m_lo < mass < m_hi where the test attaches the mass (mass > threshold in rne / nov, every mass in dyn),
+    unloaded_ok where it does not, always True in base."""
+    xp = _xp(m_lo)
+    lo = m_lo if xp is not np else np.asarray(m_lo, dtype=np.float64)
+    hi = m_hi if xp is not np else np.asarray(m_hi, dtype=np.float64)
+    ok = (unloaded_ok if xp is not np else np.asarray(unloaded_ok)) != 0
+    if mode == "base":
+        return xp.ones_like(ok)
+    inside = (lo < mass) & (hi > mass)
+    if mode == "dyn":
+        return inside
+    t = float(payload_threshold)
+    if np.ndim(mass) == 0:
+        return inside if float(mass) > t else ok
+    return xp.where(mass > t, inside, ok)
+
+
 def fp64_peak(iters: int = 4096) -> float:
     """Measured FP64 FMA throughput of the current device in FLOP/s (tcmp_fp64_peak)."""
     out = ctypes.c_double(0.0)
