@@ -306,7 +306,12 @@ int tcmp_ik_batch(int64_t n, const double *rot9, const double *trans3, const dou
  * return the one nearest to q_ref ([7][n], or [7] when ref_broadcast != 0) in the max norm (use_max_norm != 0,
  * closest_inverse_kinematics ikfast.py:172-188) or the Euclidean norm (ik_utils.select_solution :43-52).
  *   best_q [7][n], best_cost [n] (+inf when no solution survives), n_valid [n] = surviving solutions.
- * Ties keep the first solution in (free value, solver order).
+ * Ties keep the first solution in (free value, solver order).  Costs rank in numeric order and a NaN cost after every
+ * number, +inf included: a NaN in one joint of q_ref makes every cost NaN (in both norms), and the first surviving
+ * solution in (free value, solver order) is returned with best_cost = NaN and n_valid unchanged, as the drop-in's
+ * sort does.  +-inf in q_ref makes every cost +inf: again the first survivor, with best_cost = +inf.  With no
+ * survivor best_q is all zeros, best_cost +inf and n_valid 0.  A NaN limit bounds nothing (a joint passes unless it
+ * is < lo or > hi); lo > hi leaves no survivor.  A non-finite free value gives no solutions; the others are unaffected.
  * NOT the reference's order of operations: the reference takes the nearest IN-LIMIT solution first
  * (closest_inverse_kinematics) and then fails the whole grasp if that single configuration exceeds the torque limits
  * (panda_primitives.py:263), whereas this call picks the nearest solution among those that ALSO pass the torque test --

@@ -9,6 +9,7 @@
 // surviving solution and keeps the nearest feasible one -- no solution set ever leaves the SM.
 #include "ik_core.cuh"
 #include "panda_model.cuh"
+#include "select_core.cuh"
 #include "tcmp_internal.h"
 
 namespace tcmp {
@@ -18,10 +19,6 @@ namespace tcmp {
 // too few per CTA to pay for staging 16 KB.  Own copy per translation unit (no relocatable device code in the build).
 static __device__ const SinCos kSelSinCosTable[kSinCosTableSize] = {
 #include "sincos_table.inc"
-};
-
-struct JointLimits {
-    double lo[7], hi[7];
 };
 
 // One warp per pose, two dense phases (the first version ran the torque test inside the per-lane solution loop:
@@ -75,7 +72,7 @@ ik_select_kernel(int64_t n, int n_free, int free_broadcast, const double *__rest
         for (int j = 0; j < 7; ++j) ref[j] = ref_broadcast ? __ldg(q_ref + j) : __ldg(q_ref + j * n + p);
         const double tx = __ldg(trans3 + p), ty = __ldg(trans3 + n + p), tz = __ldg(trans3 + 2 * n + p);
         double wc = INFINITY;     // this lane's best feasible candidate so far: cost, key, configuration
-        int wk = 0x7fffffff, valid = 0;
+        int wk = kNoKey, valid = 0;
         double bq[7] = {0, 0, 0, 0, 0, 0, 0};
         for (int fbase = 0; fbase < n_free; fbase += 32) {
             // ---- phase A: IK + joint-limit filter for up to 32 free values ----
@@ -102,23 +99,14 @@ ik_select_kernel(int64_t n, int n_free, int free_broadcast, const double *__rest
             for (int sidx = 0; sidx < 8; ++sidx) {       // warp-synchronous: every lane walks all 8 slots
                 bool keep = sidx < cnt;
                 double q[7], c2 = 0.0, cmax = 0.0;
-                if (keep) {
-#pragma unroll
-                    for (int j = 0; j < 7; ++j) {
-                        q[j] = sols[sidx * 7 + j];
-                        keep = keep && !(q[j] < lim.lo[j]) && !(q[j] > lim.hi[j]);   // violates_limits
-                        const double d = fabs(q[j] - ref[j]);
-                        c2 += d * d;
-                        cmax = fmax(cmax, d);
-                    }
-                }
+                if (keep) keep = scan_candidate(sols + sidx * 7, ref, lim, q, c2, cmax);
                 const unsigned m = __ballot_sync(0xffffffffu, keep);
                 if (keep) {
                     // the list order is irrelevant: the KEY (f*8 + s) carries the sweep order for tie-breaks
                     double *row = cand + (ncand + __popc(m & lt_mask)) * kSelRow;
 #pragma unroll
                     for (int j = 0; j < 7; ++j) row[j] = q[j];
-                    row[7] = use_max_norm ? cmax : sqrt(c2);
+                    row[7] = candidate_cost(c2, cmax, use_max_norm);
                     row[8] = (double)(f * 8 + sidx);
                 }
                 ncand += __popc(m);
@@ -141,7 +129,7 @@ ik_select_kernel(int64_t n, int n_free, int free_broadcast, const double *__rest
                     ++valid;
                     const double cost = row[7];
                     const int key = (int)row[8];
-                    if (cost < wc || (cost == wc && key < wk)) {
+                    if (better(cost, key, wc, wk)) {
                         wc = cost;
                         wk = key;
 #pragma unroll
@@ -160,9 +148,9 @@ ik_select_kernel(int64_t n, int n_free, int free_broadcast, const double *__rest
             const int ok2 = __shfl_xor_sync(0xffffffffu, bk, off);
             const int ol = __shfl_xor_sync(0xffffffffu, bl, off);
             valid += __shfl_xor_sync(0xffffffffu, valid, off);
-            if (oc < bc || (oc == bc && ok2 < bk) || (oc == bc && ok2 == bk && ol < bl)) { bc = oc; bk = ok2; bl = ol; }
+            if (better(oc, ok2, bc, bk) || (oc == bc && ok2 == bk && ol < bl)) { bc = oc; bk = ok2; bl = ol; }
         }
-        if (lane == bl && act) {       // with no survivor every lane ties at (inf, INT_MAX): lane 0 writes zeros
+        if (lane == bl && act) {       // with no survivor every lane ties at (inf, kNoKey): lane 0 writes zeros
 #pragma unroll
             for (int j = 0; j < 7; ++j) best_q[j * n + p] = bq[j];
             best_cost[p] = bc;

@@ -362,7 +362,10 @@ def ik_select(rot9, trans3, free, q_ref, payload_mass: float = 0.0, mode: str = 
     """Goal-IK selection (tcmp_ik_select): per pose, the IK solution of the free-joint sweep that is inside the
     joint limits, passes the static torque test ``mode`` and is nearest to ``q_ref`` ([7][n] or [7]).
     Returns (best_q [7][n], best_cost [n] (+inf = none), n_valid int32 [n]); CUDA tensors in -> CUDA tensors out,
-    NumPy in -> NumPy out."""
+    NumPy in -> NumPy out.  Ties keep the first solution in (free value, solver order); a NaN cost ranks after every
+    number, so a NaN joint in ``q_ref`` returns the first surviving solution with ``best_cost`` NaN (``n_valid``
+    unchanged), and a +-inf joint the first survivor with ``best_cost`` +inf.  With no survivor: zeros, +inf, 0.  A NaN
+    limit in ``q_lo`` / ``q_hi`` bounds nothing."""
     torch = _torch()
     lib = load()
     lim = get_limits()
