@@ -131,6 +131,38 @@ int tcmp_dynamics_batch(const tcmp_model *model, int64_t n, const double *q, con
                         double *g_out, double *J_out, void *stream);
 
 /*
+ * Forward dynamics, fp64, per state: the joint accelerations a torque produces, and the inverse mass matrix -- the
+ * other direction of tcmp_rne_batch, for torque-limited kinodynamic sampling, simulation under torque saturation and
+ * operational-space control:
+ *   qdd_out  [7][n]     qdd = M(q)^-1 (tau - h(q, qd)),  h = rne(q, qd, 0)
+ *   Minv_out [7][7][n]  M(q)^-1, element (r, c) of state i at (r*7 + c)*n + i (tcmp_dynamics_batch's layout); exactly
+ *                       symmetric (one triangle computed, the mirror written)
+ * It is defined as the exact inverse of the torque test: tcmp_rne_batch(mode, ..., q, qd, qdd_out, ...,
+ * TCMP_PAYLOAD_THRESHOLD_RAW) reproduces tau on all 7 joints, within the torque contract (1e-9 N.m).
+ *   mode  TCMP_MODE_RNE: the payload is a rigid body on the flange iff m > 0 (tcmp_dynamics_batch's rule), in M and h.
+ *         TCMP_MODE_DYN: M is the arm and hand without the payload; h includes the tool-point force m g at the grasp
+ *         target for every m (negative too), as the dyn torque test applies it.
+ *         Any other mode (NOV ignores qd and qdd, BASE computes nothing) is TCMP_ERR_INVALID_ARG.
+ *   model         host pointer or NULL (compiled-in Panda), as in tcmp_dynamics_batch.
+ *   q [7][n]; qd [7][n] or NULL (zeros); tau [7][n] or NULL (zeros: free motion under gravity).
+ *   payload_mass  [n] or NULL (then payload_scalar applies to every state).
+ * M is factored as LDL^T.  Non-finite inputs:
+ *   - a NaN or infinite q (joint 1's too), qd, tau or mass of state i makes every qdd entry of state i NaN;
+ *   - M^-1 of state i is NaN iff some q (joint 1's too) or the mass is non-finite; it does not read qd or tau;
+ *   - other states are unaffected.
+ * This follows tcmp_rne_batch, which returns NaN torques for a non-finite joint 1 (no finite qdd reproduces a NaN
+ * torque), and deliberately differs from tcmp_dynamics_batch, whose M does not read q[0].
+ * A pivot that is not > 0 (a caller record whose tail has no inertia about joint 7's axis, e.g. link 7, link8 and the
+ * hand all massless and inertia-free) makes every output of the state NaN.
+ * Each output may be NULL; at least one is required when n > 0.  A bad mode, n < 0, a bad record, a NULL q with n > 0
+ * or both outputs NULL return TCMP_ERR_INVALID_ARG before any CUDA call; n == 0 otherwise returns TCMP_OK whatever
+ * the buffers.  Enqueues only: no allocation, no synchronisation, so the call can be captured in a CUDA graph.
+ */
+int tcmp_forward_dynamics_batch(const tcmp_model *model, int mode, int64_t n, const double *q, const double *qd,
+                                const double *tau, const double *payload_mass, double payload_scalar,
+                                double *qdd_out, double *Minv_out, void *stream);
+
+/*
  * Payload-mass intervals: which payload masses a state, or every waypoint of an RRT* edge, can carry within the torque
  * limits -- the inverse of the torque test, in one launch (a bisection over the mass takes ~26 torque-test launches to
  * reach 1e-6 kg over [0, 64] kg, and is wrong when the passing masses do not start at 0: a payload can pull a joint's

@@ -34,6 +34,7 @@ SIGNATURES = {
     "tcmp_model_default": (_i32, [_vp]),
     "tcmp_rne_batch_model": (_i32, [_vp, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _f64, _f64, _vp, _vp, _vp]),
     "tcmp_dynamics_batch": (_i32, [_vp, _i64, _vp, _vp, _vp, _f64, _vp, _vp, _vp, _vp, _vp]),
+    "tcmp_forward_dynamics_batch": (_i32, [_vp, _i32, _i64, _vp, _vp, _vp, _vp, _f64, _vp, _vp, _vp]),
     "tcmp_payload_interval_batch": (_i32, [_vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "tcmp_edge_payload_interval": (_i32, [_vp, _i32, _i64, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp]),
     "tcmp_edge_feasibility_model": (_i32, [_vp, _i32, _i32, _i64, _i32, _vp, _vp, _f64, _f64, _i32, _vp, _vp]),

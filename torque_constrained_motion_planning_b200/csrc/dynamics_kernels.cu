@@ -38,9 +38,6 @@ static cudaError_t launch_dyn(int64_t n, const double *q, const double *qd, cons
     return cudaGetLastError();
 }
 
-// 32-bit element offsets while the largest, 48 n + n - 1, fits (with a margin)
-static inline bool fits_int49(int64_t n) { return n < ((int64_t)0x7fffffff - ((int64_t)1 << 24)) / 49; }
-
 template <typename P>
 static cudaError_t launch_indexed_dyn(int64_t n, const double *q, const double *qd, const double *pm, double ps,
                                       double *M, double *C, double *g, double *J, const P &p, cudaStream_t st) {

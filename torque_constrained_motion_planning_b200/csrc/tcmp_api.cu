@@ -218,6 +218,21 @@ int tcmp_dynamics_batch(const tcmp_model *model, int64_t n, const double *q, con
     return TCMP_OK;
 }
 
+int tcmp_forward_dynamics_batch(const tcmp_model *model, int mode, int64_t n, const double *q, const double *qd,
+                                const double *tau, const double *payload_mass, double payload_scalar, double *qdd_out,
+                                double *Minv_out, void *stream) {
+    if (mode != TCMP_MODE_RNE && mode != TCMP_MODE_DYN)
+        return fail(TCMP_ERR_INVALID_ARG, "forward dynamics needs mode rne or dyn, got %d", mode);
+    if (n < 0) return fail(TCMP_ERR_INVALID_ARG, "negative count %lld", (long long)n);
+    if (int rc = check_model(model)) return rc;
+    if (n == 0) return TCMP_OK;
+    if (!q) return fail(TCMP_ERR_INVALID_ARG, "q is NULL");
+    if (!qdd_out && !Minv_out) return fail(TCMP_ERR_INVALID_ARG, "both outputs are NULL");
+    TCMP_CUDA(launch_forward_dynamics(model, mode, n, q, qd, tau, payload_mass, payload_scalar, qdd_out, Minv_out,
+                                      (cudaStream_t)stream));
+    return TCMP_OK;
+}
+
 static int check_payload_common(const tcmp_model *model, int mode, int64_t n) {
     if (mode < TCMP_MODE_RNE || mode > TCMP_MODE_BASE) return fail(TCMP_ERR_INVALID_ARG, "bad mode %d", mode);
     if (n < 0) return fail(TCMP_ERR_INVALID_ARG, "negative count %lld", (long long)n);

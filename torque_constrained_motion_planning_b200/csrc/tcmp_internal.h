@@ -43,10 +43,19 @@ cudaError_t launch_rne_batch_model(const tcmp_model &model, int mode, int dtype,
 void default_model_desc(tcmp_model *out);
 const char *model_desc_problem(const tcmp_model &model);
 
+// 32-bit element offsets of the [7][7][n] outputs while the largest, 48 n + n - 1, fits (with a margin)
+inline bool fits_int49(int64_t n) { return n < ((int64_t)0x7fffffff - ((int64_t)1 << 24)) / 49; }
+
 // dynamics_kernels.cu: M, C, g, J per state (any output may be NULL; model NULL = compiled-in Panda)
 cudaError_t launch_dynamics_batch(const tcmp_model *model, int64_t n, const double *q, const double *qd,
                                   const double *payload_mass, double payload_scalar, double *M_out, double *C_out,
                                   double *g_out, double *J_out, cudaStream_t st);
+
+// fd_kernels.cu: qdd = M^-1 (tau - h) and M^-1 per state (K13); mode RNE or DYN, either output may be NULL, qd / tau
+// NULL = zeros; model NULL = compiled-in Panda
+cudaError_t launch_forward_dynamics(const tcmp_model *model, int mode, int64_t n, const double *q, const double *qd,
+                                    const double *tau, const double *payload_mass, double payload_scalar,
+                                    double *qdd_out, double *Minv_out, cudaStream_t st);
 
 // payload_kernels.cu: payload-mass intervals per state (K11) and per min-jerk edge (K12); each output may be NULL,
 // mode BASE fills (-inf, +inf, 1) and reads nothing; model NULL = compiled-in Panda

@@ -526,6 +526,38 @@ def dynamics_batch(q, qd=None, payload_mass=0.0, mass_matrix: bool = True, corio
     return out
 
 
+def forward_dynamics_batch(q, qd=None, tau=None, payload_mass=0.0, mode: str = "rne", qdd: bool = True,
+                           minv: bool = False, model: Optional[InertialModel] = None):
+    """Forward dynamics per state (tcmp_forward_dynamics_batch), fp64: the joint accelerations
+    qdd = M(q)^-1 (tau - h(q, qd)) that the torques tau produce, and the inverse mass matrix M^-1.
+    q ``[7][n]``; qd, tau ``[7][n]`` or None (zeros); payload_mass scalar or ``[n]``.  mode "rne": the payload is a
+    rigid body on the flange iff m > 0; "dyn": M is the arm alone and the payload a tool-point force m g.  The result
+    inverts the torque test: torque_test_batch(q, qd, qdd, m, mode=mode, payload_threshold=0) returns tau.
+    Returns ``{"qdd": [7][n], "Minv": [7][7][n]}`` with None for what was not requested.  A non-finite q or mass makes
+    the state's outputs NaN, a non-finite qd or tau its qdd (include/tcmp.h).  CUDA tensors in -> CUDA tensors out,
+    NumPy in -> NumPy out."""
+    if not (qdd or minv):
+        raise ValueError("nothing to compute")
+    torch = _torch()
+    lib = load()
+    host = not _is_cuda_tensor(q)
+    dev = torch.device("cuda", torch.cuda.current_device()) if host else q.device
+    n = int(q.shape[1])
+    scalar, pm = (float(payload_mass), None) if np.ndim(payload_mass) == 0 else (0.0, payload_mass)
+    with torch.cuda.device(dev):
+        qt = _as_dev(q, "f64", (7, n), dev)
+        qdt = _as_dev(qd, "f64", (7, n), dev)
+        taut = _as_dev(tau, "f64", (7, n), dev)
+        pmt = _as_dev(pm, "f64", (n,), dev)
+        out = {"qdd": torch.empty((7, n), dtype=torch.float64, device=dev) if qdd else None,
+               "Minv": torch.empty((7, 7, n), dtype=torch.float64, device=dev) if minv else None}
+        check(lib.tcmp_forward_dynamics_batch(_mptr(model), MODE[mode], n, _ptr(qt), _ptr(qdt), _ptr(taut), _ptr(pmt),
+                                              scalar, _ptr(out["qdd"]), _ptr(out["Minv"]), _stream_ptr()))
+    if host:
+        return {k: None if v is None else v.cpu().numpy() for k, v in out.items()}
+    return out
+
+
 def _interval_outputs(torch, n, dev):
     return (torch.empty((n,), dtype=torch.float64, device=dev), torch.empty((n,), dtype=torch.float64, device=dev),
             torch.empty((n,), dtype=torch.uint8, device=dev))
