@@ -163,6 +163,51 @@ int tcmp_forward_dynamics_batch(const tcmp_model *model, int mode, int64_t n, co
                                 double *qdd_out, double *Minv_out, void *stream);
 
 /*
+ * Forward-dynamics rollouts, fp64: n rollouts of n_steps fixed steps of dt each, integrating qdd = f(q, qd) under a
+ * torque, in one launch -- propagation for torque-limited kinodynamic planning and simulation under torque saturation,
+ * with the first step that leaves the joint or velocity limits.
+ *   Dynamics: f(q, v) is tcmp_forward_dynamics_batch's qdd for the same model, mode (RNE or DYN only), payload rule
+ *     and non-finite rule, with the step's torque.
+ *   Torque (zero-order hold): tau is [7][n] and held for every step when tau_per_step == 0; when tau_per_step != 0 it
+ *     is [n_steps][7][n] and step k uses slice k for all four stages.  NULL means zero torque (free motion under
+ *     gravity).
+ *   Integrator: classical RK4 in exactly this order of operations (h2 = 0.5 * dt, h6 = dt / 6.0, once per call):
+ *       a1 = f(q, v)
+ *       q2 = q + h2*v;   v2 = v + h2*a1;   a2 = f(q2, v2)
+ *       q3 = q + h2*v2;  v3 = v + h2*a2;   a3 = f(q3, v3)
+ *       q4 = q + dt*v3;  v4 = v + dt*a3;   a4 = f(q4, v4)
+ *       q' = q + h6*(((v  + 2*v2) + 2*v3) + v4)
+ *       v' = v + h6*(((a1 + 2*a2) + 2*a3) + a4)
+ *     (the device may contract a product and a sum into one FMA).
+ *   q0 [7][n]; qd0 [7][n] or NULL (zeros); payload_mass [n] or NULL (then payload_scalar).
+ *   Outputs, each may be NULL but at least one is required when n > 0:
+ *     q_out, qd_out [7][n]: the state after n_steps steps;
+ *     q_traj_out, qd_traj_out [n_steps][7][n]: at index k the state after step k + 1, element (k, j, i) at
+ *       (k*7 + j)*n + i; the initial state is not stored;
+ *     first_violation_out [n] int32: the first index k in [0, n_steps) whose stored state fails a requested check, or
+ *       n_steps if none does (tcmp_edge_feasibility's convention).  The initial state is not checked.  With no check
+ *       requested it is n_steps.  The rollout always runs all n_steps: outputs after a violation are still defined.
+ *   Limits, host arrays of 7 copied into the launch parameters (as tcmp_collision_batch):
+ *     q_lo_host and q_hi_host are given together or both NULL; a stored state passes the position check iff
+ *     lo <= q <= hi on every joint.  qd_max_host may be NULL; a stored state passes the velocity check iff
+ *     |qd| <= qd_max on every joint.  A NaN in a checked quantity is a violation.  This deliberately differs from the
+ *     "NaN passes" rule of the torque and collision tests, which follows their reference: a rollout has no reference,
+ *     and a NaN state is never executable.
+ *   Non-finite inputs: a non-finite q0 or mass makes the whole rollout NaN; a non-finite qd0 or tau makes qdd NaN from
+ *   the first stage it enters, so every state after it is NaN too.  Other rollouts are unaffected.
+ * A mode other than RNE or DYN, n < 0, n_steps < 1, a dt that is not finite and > 0, a bad record, a NULL q0 with
+ * n > 0, no output at all, only one of q_lo_host / q_hi_host, a NaN limit or a qd_max < 0 return TCMP_ERR_INVALID_ARG
+ * before any CUDA call; n == 0 otherwise returns TCMP_OK whatever the buffers.  Enqueues only: no allocation, no
+ * synchronisation, so the call can be captured in a CUDA graph.  Offsets are 32-bit while 7 n n_steps fits in 31 bits
+ * and 64-bit beyond.
+ */
+int tcmp_rollout_batch(const tcmp_model *model, int mode, int64_t n, int n_steps, double dt, const double *q0,
+                       const double *qd0, const double *tau, int tau_per_step, const double *payload_mass,
+                       double payload_scalar, const double *q_lo_host, const double *q_hi_host,
+                       const double *qd_max_host, double *q_out, double *qd_out, double *q_traj_out,
+                       double *qd_traj_out, int32_t *first_violation_out, void *stream);
+
+/*
  * Payload-mass intervals: which payload masses a state, or every waypoint of an RRT* edge, can carry within the torque
  * limits -- the inverse of the torque test, in one launch (a bisection over the mass takes ~26 torque-test launches to
  * reach 1e-6 kg over [0, 64] kg, and is wrong when the passing masses do not start at 0: a payload can pull a joint's

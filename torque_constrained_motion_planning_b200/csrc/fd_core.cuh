@@ -101,6 +101,38 @@ template <typename T, typename Out> TCMP_FN void ldl_inverse(T (&A)[28], const T
         }
 }
 
+// The steps of one forward-dynamics evaluation, shared by K13 (fd_state below) and K14's RK4 stages
+// (rollout_core.cuh).
+// sin / cos of joints 2..7: the table where every angle allows it, libm otherwise.
+template <bool GLOBAL>
+TCMP_FN void fd_sincos(const double (&qs)[7], double (&s)[7], double (&c)[7], const SinCos *__restrict__ tab) {
+    if (!sincos6_table<GLOBAL>(qs, s, c, tab)) {
+#pragma unroll
+        for (int j = 1; j < 7; ++j) sincos_t<double>(qs[j], &s[j], &c[j]);
+    }
+}
+
+// M = L D L^T into m, and inv_d = D^-1 -- all NaN when bad_q is NaN (a non-finite q or mass) or a pivot is not > 0.
+template <typename P>
+TCMP_FN void fd_factor(const double (&s)[7], const double (&c)[7], const P &p, double mp, double bad_q,
+                       TriOut<double> &m, double (&inv_d)[7]) {
+    const bool ok = ldl_columns<0>(s, c, p, mp, m, inv_d) && bad_q == 0.0;
+#pragma unroll
+    for (int j = 0; j < 7; ++j) inv_d[j] = ok ? inv_d[j] : double(NAN);
+}
+
+// b <- (b - h) + bad_v with h = rne(q, qd, 0): tau in, the right-hand side of M qdd = tau - h out; bad_v (NaN for a
+// non-finite qd or tau) poisons every entry.
+template <bool TOOL, typename P>
+TCMP_FN void fd_bias(const double (&s)[7], const double (&c)[7], double q0, const double (&vs)[7], double mp, double mt,
+                     double bad_v, const P &p, double (&b)[7]) {
+    double h[7];
+    const double zero[7] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    rne_body<double, true, TOOL, P>(s, c, vs, zero, mp, mt, h, p, gravity_for(q0));
+#pragma unroll
+    for (int j = 0; j < 7; ++j) b[j] = (b[j] - h[j]) + bad_v;
+}
+
 // Load state i, solve, store.  TOOL: dyn (M without the payload, h with the tool-point force m g for every m); else
 // rne (the payload a rigid body on the flange iff m > 0, in M and h).  qd / tau NULL = zeros.  Either output may be
 // NULL (uniform branches; qdd is stored before M^-1 is formed, so it is the same with or without it).
@@ -126,23 +158,14 @@ TCMP_FN void fd_state(I n, I i, const double *__restrict__ q, const double *__re
         bad_q += qs[j] * 0.0;
         bad_v += vs[j] * 0.0 + b[j] * 0.0;
     }
-    if (!sincos6_table<GLOBAL>(qs, s, c, tab)) {
-#pragma unroll
-        for (int j = 1; j < 7; ++j) sincos_t<double>(qs[j], &s[j], &c[j]);
-    }
+    fd_sincos<GLOBAL>(qs, s, c, tab);
     const double mp = TOOL ? 0.0 : (mass > 0.0 ? mass : 0.0);   // TCMP_PAYLOAD_THRESHOLD_RAW, as tcmp_dynamics_batch
     const double mt = TOOL ? mass : 0.0;
     TriOut<double> m;
     double inv_d[7];
-    const bool ok = ldl_columns<0>(s, c, p, mp, m, inv_d) && bad_q == 0.0;
-#pragma unroll
-    for (int j = 0; j < 7; ++j) inv_d[j] = ok ? inv_d[j] : double(NAN);
+    fd_factor<P>(s, c, p, mp, bad_q, m, inv_d);
     if (qdd_out) {
-        double h[7];
-        const double zero[7] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
-        rne_body<double, true, TOOL, P>(s, c, vs, zero, mp, mt, h, p, gravity_for(qs[0]));
-#pragma unroll
-        for (int j = 0; j < 7; ++j) b[j] = (b[j] - h[j]) + bad_v;
+        fd_bias<TOOL, P>(s, c, qs[0], vs, mp, mt, bad_v, p, b);
         ldl_solve(m.A, inv_d, b);
 #pragma unroll
         for (int j = 0; j < 7; ++j) DynOut<I>::put(qdd_out + (I)j * n + i, b[j]);

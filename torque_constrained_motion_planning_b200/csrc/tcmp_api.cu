@@ -233,6 +233,35 @@ int tcmp_forward_dynamics_batch(const tcmp_model *model, int mode, int64_t n, co
     return TCMP_OK;
 }
 
+int tcmp_rollout_batch(const tcmp_model *model, int mode, int64_t n, int n_steps, double dt, const double *q0,
+                       const double *qd0, const double *tau, int tau_per_step, const double *payload_mass,
+                       double payload_scalar, const double *q_lo_host, const double *q_hi_host,
+                       const double *qd_max_host, double *q_out, double *qd_out, double *q_traj_out,
+                       double *qd_traj_out, int32_t *first_violation_out, void *stream) {
+    if (mode != TCMP_MODE_RNE && mode != TCMP_MODE_DYN)
+        return fail(TCMP_ERR_INVALID_ARG, "rollouts need mode rne or dyn, got %d", mode);
+    if (n < 0) return fail(TCMP_ERR_INVALID_ARG, "negative count %lld", (long long)n);
+    if (n_steps < 1) return fail(TCMP_ERR_INVALID_ARG, "n_steps must be >= 1, got %d", n_steps);
+    if (!(dt > 0.0 && dt < INFINITY)) return fail(TCMP_ERR_INVALID_ARG, "dt must be finite and > 0");
+    if (int rc = check_model(model)) return rc;
+    if ((q_lo_host == nullptr) != (q_hi_host == nullptr))
+        return fail(TCMP_ERR_INVALID_ARG, "q_lo and q_hi must both be given or both be NULL");
+    for (int j = 0; j < 7; ++j) {
+        if (q_lo_host && (q_lo_host[j] != q_lo_host[j] || q_hi_host[j] != q_hi_host[j]))
+            return fail(TCMP_ERR_INVALID_ARG, "NaN joint limit on joint %d", j);
+        if (qd_max_host && !(qd_max_host[j] >= 0.0))
+            return fail(TCMP_ERR_INVALID_ARG, "qd_max[%d] must be >= 0 (and not NaN)", j);
+    }
+    if (n == 0) return TCMP_OK;
+    if (!q0) return fail(TCMP_ERR_INVALID_ARG, "q0 is NULL");
+    if (!q_out && !qd_out && !q_traj_out && !qd_traj_out && !first_violation_out)
+        return fail(TCMP_ERR_INVALID_ARG, "every output is NULL");
+    TCMP_CUDA(launch_rollout(model, mode, n, n_steps, dt, q0, qd0, tau, tau_per_step, payload_mass, payload_scalar,
+                             q_lo_host, q_hi_host, qd_max_host, q_out, qd_out, q_traj_out, qd_traj_out,
+                             first_violation_out, (cudaStream_t)stream));
+    return TCMP_OK;
+}
+
 static int check_payload_common(const tcmp_model *model, int mode, int64_t n) {
     if (mode < TCMP_MODE_RNE || mode > TCMP_MODE_BASE) return fail(TCMP_ERR_INVALID_ARG, "bad mode %d", mode);
     if (n < 0) return fail(TCMP_ERR_INVALID_ARG, "negative count %lld", (long long)n);

@@ -57,6 +57,14 @@ cudaError_t launch_forward_dynamics(const tcmp_model *model, int mode, int64_t n
                                     const double *tau, const double *payload_mass, double payload_scalar,
                                     double *qdd_out, double *Minv_out, cudaStream_t st);
 
+// rollout_kernels.cu: RK4 forward-dynamics rollouts (K14); mode RNE or DYN, qd0 / tau NULL = zeros, limits are host
+// arrays of 7 (NULL = not checked), each output may be NULL; model NULL = compiled-in Panda
+cudaError_t launch_rollout(const tcmp_model *model, int mode, int64_t n, int n_steps, double dt, const double *q0,
+                           const double *qd0, const double *tau, int tau_per_step, const double *payload_mass,
+                           double payload_scalar, const double *q_lo, const double *q_hi, const double *qd_max,
+                           double *q_out, double *qd_out, double *q_traj_out, double *qd_traj_out,
+                           int32_t *first_violation_out, cudaStream_t st);
+
 // payload_kernels.cu: payload-mass intervals per state (K11) and per min-jerk edge (K12); each output may be NULL,
 // mode BASE fills (-inf, +inf, 1) and reads nothing; model NULL = compiled-in Panda
 cudaError_t launch_payload_interval(const tcmp_model *model, int mode, int64_t n, const double *q, const double *qd,

@@ -558,6 +558,47 @@ def forward_dynamics_batch(q, qd=None, tau=None, payload_mass=0.0, mode: str = "
     return out
 
 
+def rollout_batch(q0, qd0=None, tau=None, dt: float = 1e-3, n_steps: int = 1, payload_mass=0.0, mode: str = "rne",
+                  tau_per_step: bool = False, q_lo=None, q_hi=None, qd_max=None, trajectory: bool = False,
+                  model: Optional[InertialModel] = None):
+    """Forward-dynamics rollouts (tcmp_rollout_batch), fp64: n_steps classical RK4 steps of dt on
+    qdd = forward_dynamics_batch(q, qd, tau) from (q0, qd0), with the torque held (tau ``[7][n]``) or given per step
+    (tau_per_step, tau ``[n_steps][7][n]``); qd0 / tau None = zeros.  q_lo / q_hi (both or neither) and qd_max are 7
+    joint limits checked on every stored state (a NaN fails).  Returns ``{"q": [7][n], "qd": [7][n],
+    "q_traj": [n_steps][7][n], "qd_traj": [n_steps][7][n], "first_violation": int32 [n]}``: the final state, the state
+    after every step when ``trajectory``, and the first step whose state fails a check (n_steps if none), with None for
+    what was not requested.  CUDA tensors in -> CUDA tensors out, NumPy in -> NumPy out."""
+    if (q_lo is None) != (q_hi is None):
+        raise ValueError("q_lo and q_hi must both be given or both be None")
+    torch = _torch()
+    lib = load()
+    host = not _is_cuda_tensor(q0)
+    dev = torch.device("cuda", torch.cuda.current_device()) if host else q0.device
+    n = int(q0.shape[1])
+    n_steps = int(n_steps)
+    scalar, pm = (float(payload_mass), None) if np.ndim(payload_mass) == 0 else (0.0, payload_mass)
+    lim = [None if a is None else np.ascontiguousarray(np.broadcast_to(np.asarray(a, dtype=np.float64), (7,)))
+           for a in (q_lo, q_hi, qd_max)]
+    checked = q_lo is not None or qd_max is not None
+    with torch.cuda.device(dev):
+        q0t = _as_dev(q0, "f64", (7, n), dev)
+        qd0t = _as_dev(qd0, "f64", (7, n), dev)
+        taut = _as_dev(tau, "f64", (n_steps, 7, n) if tau_per_step else (7, n), dev)
+        pmt = _as_dev(pm, "f64", (n,), dev)
+        f64 = dict(dtype=torch.float64, device=dev)
+        out = {"q": torch.empty((7, n), **f64), "qd": torch.empty((7, n), **f64),
+               "q_traj": torch.empty((n_steps, 7, n), **f64) if trajectory else None,
+               "qd_traj": torch.empty((n_steps, 7, n), **f64) if trajectory else None,
+               "first_violation": torch.empty((n,), dtype=torch.int32, device=dev) if checked else None}
+        check(lib.tcmp_rollout_batch(_mptr(model), MODE[mode], n, n_steps, float(dt), _ptr(q0t), _ptr(qd0t),
+                                     _ptr(taut), int(bool(tau_per_step)), _ptr(pmt), scalar,
+                                     *(_nptr(a) for a in lim), _ptr(out["q"]), _ptr(out["qd"]), _ptr(out["q_traj"]),
+                                     _ptr(out["qd_traj"]), _ptr(out["first_violation"]), _stream_ptr()))
+    if host:
+        return {k: None if v is None else v.cpu().numpy() for k, v in out.items()}
+    return out
+
+
 def _interval_outputs(torch, n, dev):
     return (torch.empty((n,), dtype=torch.float64, device=dev), torch.empty((n,), dtype=torch.float64, device=dev),
             torch.empty((n,), dtype=torch.uint8, device=dev))
