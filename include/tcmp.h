@@ -208,6 +208,58 @@ int tcmp_rollout_batch(const tcmp_model *model, int mode, int64_t n, int n_steps
                        double *qd_traj_out, int32_t *first_violation_out, void *stream);
 
 /*
+ * Closed-loop tracking rollouts, fp64: will the arm execute a planned trajectory?  n rollouts of n_steps steps in one
+ * launch, in which a computed-torque controller follows a piecewise-quintic reference, its torque saturates at the
+ * model's limits, and the result drives tcmp_rollout_batch's plant -- under a payload the controller does not know,
+ * an initial-state error and a finite control rate.
+ *   Reference: n_seg quintic segments of unit duration, tcmp_traj_feasibility's coefficient order (a0..a5 per joint).
+ *     coeffs_broadcast != 0: one [n_seg][7][6] trajectory shared by every rollout; else [n_seg][7][6][n], element
+ *     (s, j, c, i) at ((s*7 + j)*6 + c)*n + i.  For t < n_seg: s = (int)t, u = t - s, and
+ *       x = c0 + u*(c1 + u*(c2 + u*(c3 + u*(c4 + u*c5))))
+ *       v = c1 + u*(2*c2 + u*(3*c3 + u*(4*c4 + u*(5*c5))))
+ *       a = 2*c2 + u*(6*c3 + u*(12*c4 + u*(20*c5)))
+ *     For t >= n_seg the end is held: x as above on segment n_seg - 1 at u = 1.0, v = a = 0.
+ *   Control (zero-order hold at dt), step k = 0 .. n_steps - 1, t_k = (double)k * dt, state (q, qd) before the step:
+ *       a_cmd = (a(t_k) + kp*(x(t_k) - q)) + kd*(v(t_k) - qd)                      per joint
+ *       tau_cmd = the inverse dynamics at (q, qd, a_cmd) with the controller's mass m_c: rne mode, the payload is a
+ *                 rigid body on the flange iff m_c > 0; dyn mode, the tool-point force m_c g for every m_c
+ *                 (tcmp_forward_dynamics_batch's rule; tcmp_rne_batch with threshold 0 gives the same torques)
+ *       tau_j = |tau_cmd_j| > L_j ? copysign(L_j, tau_cmd_j) : tau_cmd_j             on all 7 joints (joint 7 too,
+ *                 which the torque test never checks); L = the model's torque_limit[7]; a NaN passes unchanged
+ *     then one tcmp_rollout_batch step from (q, qd) with tau held and the plant's mass m_p: bit-identical, in a host
+ *     build, to tcmp_rollout_batch(n_steps = 1, tau).  (The device may contract a product and a sum into one FMA.)
+ *   kp_host, kd_host: host arrays of 7 gains, copied into the launch parameters.
+ *   payload_mass [n] or NULL (then payload_scalar): m_p, the plant's.  ctrl_payload_mass [n] or NULL (then
+ *     ctrl_payload_scalar): m_c, the controller's.  Only the payload mass differs between the two models.
+ *   q0, qd0 [7][n]; NULL means x(0) / v(0) of each rollout's reference.  This deliberately differs from
+ *     tcmp_rollout_batch, where NULL means zeros: tracking starts on the reference unless an offset is given.
+ *   Outputs, each may be NULL but at least one is required when n > 0:
+ *     q_out, qd_out [7][n]: the state after n_steps steps;
+ *     q_traj_out, qd_traj_out [n_steps][7][n]: at index k the state after step k + 1 (tcmp_rollout_batch's);
+ *     tau_traj_out [n_steps][7][n]: at index k the applied (saturated) torque of step k;
+ *     first_violation_out [n] int32: tcmp_rollout_batch's joint- and velocity-limit check, unchanged (a NaN fails);
+ *     first_saturation_out [n] int32: the first k at which some |tau_cmd_j| > L_j, or n_steps if none;
+ *     max_err_out [n]: the maximum over k and all 7 joints of |q_{k+1,j} - x_j(t_{k+1})| on the stored states; NaN
+ *       if any such term is NaN.
+ *   Limits: as tcmp_rollout_batch.
+ *   Non-finite inputs: tcmp_rollout_batch's rules for q0, qd0 and m_p.  A non-finite coefficient or m_c makes tau NaN
+ *   from the step that first reads it (a coefficient is read in the segment it belongs to), so the rollout is NaN
+ *   from then on.  Other rollouts are unaffected.
+ * Rejected with TCMP_ERR_INVALID_ARG before any CUDA call: whatever tcmp_rollout_batch rejects (but q0 may be NULL),
+ * n_seg < 1, NULL kp_host or kd_host, a gain that is negative or not finite, and, with n > 0, NULL coeffs.  n == 0
+ * otherwise returns TCMP_OK whatever the buffers.  Enqueues only: no allocation, no synchronisation, so the call can
+ * be captured in a CUDA graph.  Offsets are 32-bit while 7 n n_steps and (per-rollout coefficients) 42 n_seg n fit in
+ * 31 bits, and 64-bit beyond.
+ */
+int tcmp_track_batch(const tcmp_model *model, int mode, int64_t n, int n_steps, double dt, int n_seg,
+                     const double *coeffs, int coeffs_broadcast, const double *q0, const double *qd0,
+                     const double *kp_host, const double *kd_host, const double *payload_mass, double payload_scalar,
+                     const double *ctrl_payload_mass, double ctrl_payload_scalar, const double *q_lo_host,
+                     const double *q_hi_host, const double *qd_max_host, double *q_out, double *qd_out,
+                     double *q_traj_out, double *qd_traj_out, double *tau_traj_out, int32_t *first_violation_out,
+                     int32_t *first_saturation_out, double *max_err_out, void *stream);
+
+/*
  * Payload-mass intervals: which payload masses a state, or every waypoint of an RRT* edge, can carry within the torque
  * limits -- the inverse of the torque test, in one launch (a bisection over the mass takes ~26 torque-test launches to
  * reach 1e-6 kg over [0, 64] kg, and is wrong when the passing masses do not start at 0: a payload can pull a joint's

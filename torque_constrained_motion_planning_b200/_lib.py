@@ -37,6 +37,8 @@ SIGNATURES = {
     "tcmp_forward_dynamics_batch": (_i32, [_vp, _i32, _i64, _vp, _vp, _vp, _vp, _f64, _vp, _vp, _vp]),
     "tcmp_rollout_batch": (_i32, [_vp, _i32, _i64, _i32, _f64, _vp, _vp, _vp, _i32, _vp, _f64, _vp, _vp, _vp, _vp, _vp, _vp,
                                   _vp, _vp, _vp]),
+    "tcmp_track_batch": (_i32, [_vp, _i32, _i64, _i32, _f64, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _f64, _vp, _f64,
+                                _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "tcmp_payload_interval_batch": (_i32, [_vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "tcmp_edge_payload_interval": (_i32, [_vp, _i32, _i64, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp]),
     "tcmp_edge_feasibility_model": (_i32, [_vp, _i32, _i32, _i64, _i32, _vp, _vp, _f64, _f64, _i32, _vp, _vp]),

@@ -107,36 +107,48 @@ struct RollArgs {
     int32_t *first_violation;
 };
 
+// K14's torque source: the initial state from q0 / qd0 (qd0 NULL = zeros), and the torque held ([7][n]) or given per
+// step ([n_steps][7][n]), NULL = zero; nothing else observed.  rollout_state calls a policy's init once, torque before
+// each step (it leaves the step's torque in the kRollU rows), observe on each stored state and finish at the end, each
+// with the scratch column.  K15 (track_core.cuh) supplies a controller instead.
+struct RollHeldTorque {
+    template <typename I> TCMP_FN void init(const RollArgs &a, I i, double *__restrict__ S, int ld) {
+        const I n = (I)a.n;
+#pragma unroll
+        for (int j = 0; j < 7; ++j) {
+            S[(kRollQ + j) * ld] = roll_load<I>(a.q0 + (I)j * n + i);
+            S[(kRollV + j) * ld] = a.qd0 ? roll_load<I>(a.qd0 + (I)j * n + i) : 0.0;
+            S[(kRollU + j) * ld] = 0.0;
+        }
+    }
+    template <typename I> TCMP_FN void torque(const RollArgs &a, int k, I i, double *__restrict__ S, int ld) {
+        if (a.tau && (a.tau_per_step || k == 0)) {
+            const I n = (I)a.n;
+            const double *t = a.tau_per_step ? a.tau + (I)k * 7 * n : a.tau;
+#pragma unroll
+            for (int j = 0; j < 7; ++j) S[(kRollU + j) * ld] = roll_load<I>(t + (I)j * n + i);
+        }
+    }
+    template <typename I> TCMP_FN void observe(int, I, const double (&)[7], double *__restrict__, int) {}
+    template <typename I> TCMP_FN void finish(I, double *__restrict__, int) {}
+};
+
 // Rollout i.  The first violation is n_steps when no stored state fails (or nothing is checked).
-template <typename I, bool TOOL, typename P, bool GLOBAL = false>
+template <typename I, bool TOOL, typename P, bool GLOBAL = false, typename Pol = RollHeldTorque>
 TCMP_FN void rollout_state(const RollArgs &args, I i, const P &p, const SinCos *__restrict__ tab,
-                           double *__restrict__ S, int ld) {
+                           double *__restrict__ S, int ld, Pol pol = Pol()) {
 #define TCMP_ROW(r) S[(r) * ld]
     {
         const RollArgs &a = args;
-        const I n = (I)a.n;
         const double mass = a.payload_mass ? roll_load<I>(a.payload_mass + i) : a.payload_scalar;
         TCMP_ROW(kRollMass) = mass;
         TCMP_ROW(kRollZero) = 0.0;   // all-zero bits: roll_fresh's offset
-#pragma unroll
-        for (int j = 0; j < 7; ++j) {
-            TCMP_ROW(kRollQ + j) = roll_load<I>(a.q0 + (I)j * n + i);
-            TCMP_ROW(kRollV + j) = a.qd0 ? roll_load<I>(a.qd0 + (I)j * n + i) : 0.0;
-            TCMP_ROW(kRollU + j) = 0.0;
-        }
+        pol.init(a, i, S, ld);
     }
     int first = -1;
 #pragma unroll 1
     for (int k = 0; k < args.n_steps; ++k) {
-        {
-            const RollArgs &a = args;
-            if (a.tau && (a.tau_per_step || k == 0)) {
-                const I n = (I)a.n;
-                const double *t = a.tau_per_step ? a.tau + (I)k * 7 * n : a.tau;
-#pragma unroll
-                for (int j = 0; j < 7; ++j) TCMP_ROW(kRollU + j) = roll_load<I>(t + (I)j * n + i);
-            }
-        }
+        pol.torque(args, k, i, S, ld);
         double qs[7], vs[7];
 #pragma unroll
         for (int j = 0; j < 7; ++j) {
@@ -209,6 +221,7 @@ TCMP_FN void rollout_state(const RollArgs &args, I i, const P &p, const SinCos *
             for (int j = 0; j < 7; ++j) DynOut<I>::put(a.qd_traj + ((I)k * 7 + j) * n + i, vs[j]);
         }
         if (first < 0 && !roll_state_ok(qs, vs, a.lim)) first = k;
+        pol.observe(k, i, qs, S, ld);
     }
     const RollArgs &a = args;
     const I n = (I)a.n;
@@ -218,6 +231,7 @@ TCMP_FN void rollout_state(const RollArgs &args, I i, const P &p, const SinCos *
         if (a.qd_out) DynOut<I>::put(a.qd_out + (I)j * n + i, TCMP_ROW(kRollV + j));
     }
     if (a.first_violation) a.first_violation[i] = first < 0 ? a.n_steps : first;
+    pol.finish(i, S, ld);
 #undef TCMP_ROW
 }
 

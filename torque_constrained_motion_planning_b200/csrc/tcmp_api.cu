@@ -233,11 +233,9 @@ int tcmp_forward_dynamics_batch(const tcmp_model *model, int mode, int64_t n, co
     return TCMP_OK;
 }
 
-int tcmp_rollout_batch(const tcmp_model *model, int mode, int64_t n, int n_steps, double dt, const double *q0,
-                       const double *qd0, const double *tau, int tau_per_step, const double *payload_mass,
-                       double payload_scalar, const double *q_lo_host, const double *q_hi_host,
-                       const double *qd_max_host, double *q_out, double *qd_out, double *q_traj_out,
-                       double *qd_traj_out, int32_t *first_violation_out, void *stream) {
+// What tcmp_rollout_batch and tcmp_track_batch reject alike.
+static int check_rollout_common(const tcmp_model *model, int mode, int64_t n, int n_steps, double dt,
+                                const double *q_lo_host, const double *q_hi_host, const double *qd_max_host) {
     if (mode != TCMP_MODE_RNE && mode != TCMP_MODE_DYN)
         return fail(TCMP_ERR_INVALID_ARG, "rollouts need mode rne or dyn, got %d", mode);
     if (n < 0) return fail(TCMP_ERR_INVALID_ARG, "negative count %lld", (long long)n);
@@ -252,6 +250,15 @@ int tcmp_rollout_batch(const tcmp_model *model, int mode, int64_t n, int n_steps
         if (qd_max_host && !(qd_max_host[j] >= 0.0))
             return fail(TCMP_ERR_INVALID_ARG, "qd_max[%d] must be >= 0 (and not NaN)", j);
     }
+    return TCMP_OK;
+}
+
+int tcmp_rollout_batch(const tcmp_model *model, int mode, int64_t n, int n_steps, double dt, const double *q0,
+                       const double *qd0, const double *tau, int tau_per_step, const double *payload_mass,
+                       double payload_scalar, const double *q_lo_host, const double *q_hi_host,
+                       const double *qd_max_host, double *q_out, double *qd_out, double *q_traj_out,
+                       double *qd_traj_out, int32_t *first_violation_out, void *stream) {
+    if (int rc = check_rollout_common(model, mode, n, n_steps, dt, q_lo_host, q_hi_host, qd_max_host)) return rc;
     if (n == 0) return TCMP_OK;
     if (!q0) return fail(TCMP_ERR_INVALID_ARG, "q0 is NULL");
     if (!q_out && !qd_out && !q_traj_out && !qd_traj_out && !first_violation_out)
@@ -259,6 +266,31 @@ int tcmp_rollout_batch(const tcmp_model *model, int mode, int64_t n, int n_steps
     TCMP_CUDA(launch_rollout(model, mode, n, n_steps, dt, q0, qd0, tau, tau_per_step, payload_mass, payload_scalar,
                              q_lo_host, q_hi_host, qd_max_host, q_out, qd_out, q_traj_out, qd_traj_out,
                              first_violation_out, (cudaStream_t)stream));
+    return TCMP_OK;
+}
+
+int tcmp_track_batch(const tcmp_model *model, int mode, int64_t n, int n_steps, double dt, int n_seg,
+                     const double *coeffs, int coeffs_broadcast, const double *q0, const double *qd0,
+                     const double *kp_host, const double *kd_host, const double *payload_mass, double payload_scalar,
+                     const double *ctrl_payload_mass, double ctrl_payload_scalar, const double *q_lo_host,
+                     const double *q_hi_host, const double *qd_max_host, double *q_out, double *qd_out,
+                     double *q_traj_out, double *qd_traj_out, double *tau_traj_out, int32_t *first_violation_out,
+                     int32_t *first_saturation_out, double *max_err_out, void *stream) {
+    if (int rc = check_rollout_common(model, mode, n, n_steps, dt, q_lo_host, q_hi_host, qd_max_host)) return rc;
+    if (n_seg < 1) return fail(TCMP_ERR_INVALID_ARG, "n_seg must be >= 1, got %d", n_seg);
+    if (!kp_host || !kd_host) return fail(TCMP_ERR_INVALID_ARG, "kp and kd are required");
+    for (int j = 0; j < 7; ++j)
+        if (!(kp_host[j] >= 0.0 && kp_host[j] < INFINITY && kd_host[j] >= 0.0 && kd_host[j] < INFINITY))
+            return fail(TCMP_ERR_INVALID_ARG, "gains of joint %d must be finite and >= 0", j);
+    if (n == 0) return TCMP_OK;
+    if (!coeffs) return fail(TCMP_ERR_INVALID_ARG, "coeffs is NULL");
+    if (!q_out && !qd_out && !q_traj_out && !qd_traj_out && !tau_traj_out && !first_violation_out &&
+        !first_saturation_out && !max_err_out)
+        return fail(TCMP_ERR_INVALID_ARG, "every output is NULL");
+    TCMP_CUDA(launch_track(model, mode, n, n_steps, dt, n_seg, coeffs, coeffs_broadcast, q0, qd0, kp_host, kd_host,
+                           payload_mass, payload_scalar, ctrl_payload_mass, ctrl_payload_scalar, q_lo_host, q_hi_host,
+                           qd_max_host, q_out, qd_out, q_traj_out, qd_traj_out, tau_traj_out, first_violation_out,
+                           first_saturation_out, max_err_out, (cudaStream_t)stream));
     return TCMP_OK;
 }
 

@@ -65,6 +65,17 @@ cudaError_t launch_rollout(const tcmp_model *model, int mode, int64_t n, int n_s
                            double *q_out, double *qd_out, double *q_traj_out, double *qd_traj_out,
                            int32_t *first_violation_out, cudaStream_t st);
 
+// track_kernels.cu: closed-loop tracking rollouts (K15); mode RNE or DYN, q0 / qd0 NULL = the reference's x(0) / v(0),
+// gains and limits are host arrays of 7 (limits NULL = not checked), each output may be NULL; model NULL = compiled-in
+// Panda
+cudaError_t launch_track(const tcmp_model *model, int mode, int64_t n, int n_steps, double dt, int n_seg,
+                         const double *coeffs, int coeffs_broadcast, const double *q0, const double *qd0,
+                         const double *kp, const double *kd, const double *payload_mass, double payload_scalar,
+                         const double *ctrl_payload_mass, double ctrl_payload_scalar, const double *q_lo,
+                         const double *q_hi, const double *qd_max, double *q_out, double *qd_out, double *q_traj_out,
+                         double *qd_traj_out, double *tau_traj_out, int32_t *first_violation_out,
+                         int32_t *first_saturation_out, double *max_err_out, cudaStream_t st);
+
 // payload_kernels.cu: payload-mass intervals per state (K11) and per min-jerk edge (K12); each output may be NULL,
 // mode BASE fills (-inf, +inf, 1) and reads nothing; model NULL = compiled-in Panda
 cudaError_t launch_payload_interval(const tcmp_model *model, int mode, int64_t n, const double *q, const double *qd,

@@ -599,6 +599,99 @@ def rollout_batch(q0, qd0=None, tau=None, dt: float = 1e-3, n_steps: int = 1, pa
     return out
 
 
+def edge_coefficients(qa, qb):
+    """The two-point min-jerk edges qa -> qb (``[7][n]`` each) that tcmp_edge_feasibility samples, as a one-segment
+    reference for track_batch: ``[1][7][6][n]`` with a0 = qa, a3..a5 = 10 A, -15 A, 6 A (A = qb - qa), the rest 0.
+    CUDA tensors in -> a CUDA tensor out, NumPy in -> NumPy out."""
+    if _is_cuda_tensor(qa):
+        torch = _torch()
+        qa_t = qa.to(torch.float64)
+        A = qb.to(device=qa.device, dtype=torch.float64) - qa_t
+        c = torch.zeros((1, 7, 6) + tuple(qa.shape[1:]), dtype=torch.float64, device=qa.device)
+        c[0, :, 0], c[0, :, 3], c[0, :, 4], c[0, :, 5] = qa_t, 10 * A, -15 * A, 6 * A
+        return c
+    qa_n = np.asarray(qa, dtype=np.float64)
+    A = np.asarray(qb, dtype=np.float64) - qa_n
+    c = np.zeros((1, 7, 6) + qa_n.shape[1:])
+    c[0, :, 0], c[0, :, 3], c[0, :, 4], c[0, :, 5] = qa_n, 10 * A, -15 * A, 6 * A
+    return c
+
+
+def track_batch(coeffs, dt: float, n_steps: int, kp, kd, q0=None, qd0=None, payload_mass=0.0, ctrl_payload_mass=None,
+                mode: str = "rne", q_lo=None, q_hi=None, qd_max=None, trajectory: bool = False, n: Optional[int] = None,
+                model: Optional[InertialModel] = None):
+    """Closed-loop tracking rollouts (tcmp_track_batch), fp64: a computed-torque controller,
+    a_cmd = a_ref + kp (x_ref - q) + kd (v_ref - qd) through the inverse dynamics with the controller's payload mass,
+    saturated at the model's torque limits on all 7 joints and held for dt, drives the RK4 plant of rollout_batch with
+    the true payload mass, for n_steps steps.
+    coeffs: the piecewise-quintic reference of unit-duration segments in traj_feasibility's order, ``[n_seg][7][6]``
+    shared by every rollout or ``[n_seg][7][6][n]`` per rollout (edge_coefficients builds edges); the end is held after
+    the last segment.  kp, kd: 7 gains >= 0 (scalars broadcast).  q0 / qd0 ``[7][n]`` or None (start on the
+    reference).  payload_mass (the plant's) and ctrl_payload_mass (the controller's; None = the same) scalar or
+    ``[n]``.  q_lo / q_hi (both or neither) and qd_max: rollout_batch's limit check.  With shared coefficients n comes
+    from the per-rollout inputs, or from ``n`` when there are none.
+    Returns ``{"q", "qd": [7][n], "q_traj", "qd_traj", "tau_traj": [n_steps][7][n], "first_violation",
+    "first_saturation": int32 [n], "max_err": [n]}``: the final state; with ``trajectory`` the state after every step
+    and the applied torque of every step; the first step whose state fails a check (when limits are given) and the
+    first step whose commanded torque exceeds a limit (n_steps if none); the largest |q - x_ref| over the stored states.
+    None for what was not requested.  CUDA tensors in -> CUDA tensors out, NumPy in -> NumPy out."""
+    if (q_lo is None) != (q_hi is None):
+        raise ValueError("q_lo and q_hi must both be given or both be None")
+    ndim = len(coeffs.shape)
+    if ndim not in (3, 4) or tuple(coeffs.shape[1:3]) != (7, 6):
+        raise ValueError("coeffs must be [n_seg][7][6] or [n_seg][7][6][n], got %s" % (tuple(coeffs.shape),))
+    n_seg = int(coeffs.shape[0])
+    per_rollout = [a for a in (q0, qd0) if a is not None]
+    per_rollout += [m for m in (payload_mass, ctrl_payload_mass) if m is not None and np.ndim(m) == 1]
+    if ndim == 4:
+        n_in = int(coeffs.shape[3])
+    elif per_rollout:
+        n_in = int(per_rollout[0].shape[-1]) if hasattr(per_rollout[0], "shape") else len(per_rollout[0])
+    elif n is not None:
+        n_in = int(n)
+    else:
+        raise ValueError("shared coefficients need a per-rollout input or n= to give the number of rollouts")
+    if n is not None and int(n) != n_in:
+        raise ValueError("n=%d does not match the inputs' %d rollouts" % (int(n), n_in))
+    n = n_in
+    torch = _torch()
+    lib = load()
+    cuda_in = [a for a in [coeffs] + per_rollout if _is_cuda_tensor(a)]
+    host = not cuda_in
+    dev = torch.device("cuda", torch.cuda.current_device()) if host else cuda_in[0].device
+    n_steps = int(n_steps)
+    scalar, pm = (float(payload_mass), None) if np.ndim(payload_mass) == 0 else (0.0, payload_mass)
+    if ctrl_payload_mass is None:
+        cscalar, cpm = scalar, pm
+    else:
+        cscalar, cpm = (float(ctrl_payload_mass), None) if np.ndim(ctrl_payload_mass) == 0 else (0.0, ctrl_payload_mass)
+    gains = [np.ascontiguousarray(np.broadcast_to(np.asarray(g, dtype=np.float64), (7,))) for g in (kp, kd)]
+    lim = [None if a is None else np.ascontiguousarray(np.broadcast_to(np.asarray(a, dtype=np.float64), (7,)))
+           for a in (q_lo, q_hi, qd_max)]
+    checked = q_lo is not None or qd_max is not None
+    with torch.cuda.device(dev):
+        ct = _as_dev(coeffs, "f64", (n_seg, 7, 6) if ndim == 3 else (n_seg, 7, 6, n), dev)
+        q0t = _as_dev(q0, "f64", (7, n), dev)
+        qd0t = _as_dev(qd0, "f64", (7, n), dev)
+        pmt = _as_dev(pm, "f64", (n,), dev)
+        cpmt = pmt if cpm is pm else _as_dev(cpm, "f64", (n,), dev)
+        f64 = dict(dtype=torch.float64, device=dev)
+        i32 = dict(dtype=torch.int32, device=dev)
+        traj = lambda: torch.empty((n_steps, 7, n), **f64) if trajectory else None
+        out = {"q": torch.empty((7, n), **f64), "qd": torch.empty((7, n), **f64), "q_traj": traj(), "qd_traj": traj(),
+               "tau_traj": traj(), "first_violation": torch.empty((n,), **i32) if checked else None,
+               "first_saturation": torch.empty((n,), **i32), "max_err": torch.empty((n,), **f64)}
+        check(lib.tcmp_track_batch(_mptr(model), MODE[mode], n, n_steps, float(dt), n_seg, _ptr(ct), int(ndim == 3),
+                                   _ptr(q0t), _ptr(qd0t), *(_nptr(g) for g in gains), _ptr(pmt), scalar, _ptr(cpmt),
+                                   cscalar, *(_nptr(a) for a in lim), _ptr(out["q"]), _ptr(out["qd"]),
+                                   _ptr(out["q_traj"]), _ptr(out["qd_traj"]), _ptr(out["tau_traj"]),
+                                   _ptr(out["first_violation"]), _ptr(out["first_saturation"]), _ptr(out["max_err"]),
+                                   _stream_ptr()))
+    if host:
+        return {k: None if v is None else v.cpu().numpy() for k, v in out.items()}
+    return out
+
+
 def _interval_outputs(torch, n, dev):
     return (torch.empty((n,), dtype=torch.float64, device=dev), torch.empty((n,), dtype=torch.float64, device=dev),
             torch.empty((n,), dtype=torch.uint8, device=dev))
